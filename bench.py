@@ -18,6 +18,8 @@ enwik8-shaped XML/wiki text, deflate format, default 1 MiB max-block (96 blocks)
 Parity gate before any number counts: the complete stream of every configuration must equal the unmodified reference's
 (sha256 in tests/golden/config_golden.npz, made by tests/golden/make_config_golden.py where the reference compiles).
 --impl reference times the reference CPU implementation on the host cores instead (no GPU work).
+--dump-outputs DIR writes the stream of the last timed step (see dump_outputs) so that two builds can be compared
+output for output; the inputs are generated from fixed seeds, so the same arguments give the same inputs.
 """
 import argparse
 import ctypes as C
@@ -241,6 +243,28 @@ def verify_stream(name, weak, data, stream, flags):
     return "inflate(stream) == input"
 
 
+DUMP_SAMPLE = 4 << 20     # stream bytes kept by --dump-outputs: 16 MB of float32 values + 32 MB of float64 positions
+
+
+def dump_outputs(out_dir, stream, checksum):
+    """The complete framed stream a caller of the timed path receives, as .npy files under out_dir:
+      stream.npy         its bytes as float32 - all of them, or DUMP_SAMPLE bytes at positions drawn with a fixed seed
+      stream_index.npy   the positions of those bytes in the stream (float64)
+      stream_sha256.npy  the 32 bytes of sha256 of the whole stream (float32), so that every byte is compared
+      checksum.npy       [stream length in bytes, adler32 / crc32 of the input the path returned] (float64)"""
+    import hashlib
+    os.makedirs(out_dir, exist_ok=True)
+    b = np.frombuffer(stream, dtype=np.uint8)
+    if len(b) <= DUMP_SAMPLE:
+        idx = np.arange(len(b))
+    else:
+        idx = np.sort(np.random.default_rng(0x5A17D).choice(len(b), DUMP_SAMPLE, replace=False))
+    np.save(os.path.join(out_dir, "stream.npy"), b[idx].astype(np.float32))
+    np.save(os.path.join(out_dir, "stream_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "stream_sha256.npy"), np.frombuffer(hashlib.sha256(stream).digest(), dtype=np.uint8).astype(np.float32))
+    np.save(os.path.join(out_dir, "checksum.npy"), np.array([len(b), checksum], dtype=np.float64))
+
+
 def run_workload(args, name, weak, steps, warmup, env, headline):
     """One workload on all ranks.  Returns the result dict on rank 0 (None elsewhere)."""
     torch, dist, z, L, rank, world, local = env["torch"], env["dist"], env["z"], env["L"], env["rank"], env["world"], env["local"]
@@ -272,12 +296,6 @@ def run_workload(args, name, weak, steps, warmup, env, headline):
 
     for _ in range(warmup):
         step(False)
-    verified, stream_sha = None, None
-    if rank == 0:
-        import hashlib
-        stream = runner.final_stream()
-        verified = verify_stream(name, weak, data, stream, w["flags"])
-        stream_sha = hashlib.sha256(stream).hexdigest()
     times, l0 = [], L.zultra_cuda_launch_count()
     bsum = {}
     if headline and env.get("sampler"):
@@ -289,6 +307,14 @@ def run_workload(args, name, weak, steps, warmup, env, headline):
     if headline and env.get("sampler"):
         env["sampler"].mark_end()
     launches = L.zultra_cuda_launch_count() - l0
+    verified, stream_sha = None, None
+    if rank == 0:      # the stream of the last timed step
+        import hashlib
+        stream = runner.final_stream()
+        verified = verify_stream(name, weak, data, stream, w["flags"])
+        stream_sha = hashlib.sha256(stream).hexdigest()
+        if headline and args.dump_outputs:
+            dump_outputs(args.dump_outputs, stream, runner.checksum)
     t = torch.tensor([sum(times)], dtype=torch.float64, device="cuda")
     lt = torch.tensor([float(launches)], dtype=torch.float64, device="cuda")
     per_rank = None
@@ -374,7 +400,10 @@ def main():
     ap.add_argument("--strong-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-profile", action="store_true", help="no per-kernel CUDA events in the timed steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the stream of the last timed step of the headline workload to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0 or args.strong_steps < 1:
+        ap.error("--steps and --strong-steps must be at least 1, --warmup at least 0")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         run_reference(args, rank, world)

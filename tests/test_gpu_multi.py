@@ -2,7 +2,7 @@
 stitch.  The single-device tests drive the chunk C-ABI with two contexts on one GPU standing in for two ranks; the
 multi-device tests (skipped on a 1-GPU box) go through the library's own in-process path - zultra_cuda_ctx_set_devices /
 ZULTRA_CUDA_DEVICES behind zultra_cuda_compress_blocks, zultra_memory_compress, the streaming API and the CLI.
-Everything is compared byte for byte with the compiled reference (oracle/_ref)."""
+Everything is compared byte for byte with the reference's outputs (fingerprints in tests/golden/ref_golden.npz)."""
 import os
 import subprocess
 import zlib
@@ -10,6 +10,7 @@ import zlib
 import numpy as np
 import pytest
 
+import cases
 from zultra_b200 import shard, synth
 
 pytestmark = pytest.mark.gpu
@@ -26,23 +27,11 @@ def _ngpu(z):
     return z.load().zultra_cuda_device_count()
 
 
-def _mixed(seed):
-    rng = np.random.default_rng(seed)
-    return np.concatenate([synth.enwik(700000, seed=seed), rng.integers(0, 256, size=300000).astype(np.uint8), synth.mozilla(900000, seed=seed + 1),
-                           np.zeros(200000, dtype=np.uint8), rng.integers(0, 256, size=150000).astype(np.uint8), synth.enwik(450000, seed=seed + 2)])
-
-
-def _strip(stream, flags):
-    hdr = 0 if flags == 0 else (2 if flags == 1 else 10)
-    ftr = 0 if flags == 0 else (4 if flags == 1 else 8)
-    return stream[hdr:len(stream) - ftr]
-
-
 @pytest.mark.parametrize("world,block,g", [(2, 131072, 2), (3, 65536, 1), (4, 262144, 1)])
-def test_chunk_abi_two_contexts_stitch_vs_compiled_reference(z, ref, world, block, g):
+def test_chunk_abi_two_contexts_stitch_vs_compiled_reference(z, world, block, g):
     """zultra_cuda_chunks_prepare / _emit / zultra_cuda_stitch_device: `world` contexts on this GPU play the ranks."""
     import torch
-    data = _mixed(71 + world)
+    data = cases.mixed(71 + world)
     dev_in = torch.from_numpy(data).cuda()
     plan = shard.plan_chunks(len(data), block, world, g=g)
     ctxs = [z.CudaCtx() for _ in range(world)]
@@ -65,8 +54,7 @@ def test_chunk_abi_two_contexts_stitch_vs_compiled_reference(z, ref, world, bloc
             dst = torch.zeros((total + 7) // 8 + 8, dtype=torch.uint8, device="cuda")
             ctxs[0].stitch_device(dst.data_ptr(), src, dbit, nb)
             got = dst[: (total + 7) // 8].cpu().numpy().tobytes()
-            want = ref.compress(data, flags=flags, block=block)
-            assert got == _strip(want, flags), (world, block, flags)
+            assert cases.same_as_ref("mixed%d/%s/b%d/body" % (71 + world, cases.FMT[flags], block), got), (world, block, flags)
             ck = cks[0]
             for j in range(1, len(plan)):
                 ck = z.load().zultra_cuda_checksum_combine(flags, ck, cks[j], plan[j][1] - plan[j][0])
@@ -107,22 +95,21 @@ def test_stitch_device_random_parts(z):
     assert dst[: (pos + 7) // 8].cpu().numpy().tobytes() == want and start < 8
 
 
-def test_multi_device_compress_blocks_vs_compiled_reference(z, ref):
+def test_multi_device_compress_blocks_vs_compiled_reference(z):
     """The in-library multi-GPU path on every device count the box has."""
     n = _ngpu(z)
     if n < 2:
         pytest.skip("needs >= 2 GPUs")
-    data = _mixed(91)
+    data = cases.mixed(91)
     for ndev in sorted({2, min(n, 3), n}):
         for block in (65536, 262144):
             c = z.CudaCtx(0)
             try:
                 assert c.set_devices(ndev) == ndev
                 for flags in (0, 1, 2):
-                    want = ref.compress(data, flags=flags, block=block)
                     got, bits, ck = c.compress_blocks(data, block=block, finalize=1, flags=flags)
                     assert c.counters()["devices"] == ndev
-                    assert got == _strip(want, flags), (ndev, block, flags)
+                    assert cases.same_as_ref("mixed91/%s/b%d/body" % (cases.FMT[flags], block), got), (ndev, block, flags)
                     if flags == 1:
                         assert ck == zlib.adler32(data.tobytes())
                     if flags == 2:
@@ -131,27 +118,26 @@ def test_multi_device_compress_blocks_vs_compiled_reference(z, ref):
                 cut = 6 * block
                 a, abits, ack = c.compress_blocks(data[:cut], block=block, finalize=0, flags=2)
                 b, bbits, bck = c.compress_blocks(data[cut:], hist=data[cut - 32768:cut].copy(), block=block, finalize=1, in_bits=abits & 7, flags=2, checksum=ack)
-                want = _strip(ref.compress(data, flags=2, block=block), 2)
                 joined = bytearray(a)
                 if abits & 7:
                     joined[-1] |= b[0]
                     joined += b[1:]
                 else:
                     joined += b
-                assert bytes(joined) == want and bck == zlib.crc32(data.tobytes())
+                assert cases.same_as_ref("mixed91/gzip/b%d/body" % block, bytes(joined)) and bck == zlib.crc32(data.tobytes())
             finally:
                 c.close()
 
 
-def test_multi_device_public_api_and_cli_vs_compiled_reference(z, ref, monkeypatch, tmp_path):
+def test_multi_device_public_api_and_cli_vs_compiled_reference(z, monkeypatch, tmp_path):
     """ZULTRA_CUDA_DEVICES: zultra_memory_compress, the streaming API and the CLI on all GPUs == the reference."""
     n = _ngpu(z)
     if n < 2:
         pytest.skip("needs >= 2 GPUs")
     monkeypatch.setenv("ZULTRA_CUDA_DEVICES", str(n))
     data = synth.mix(24 << 20, seed=123, seg_lo=1 << 20, seg_hi=5 << 20)
-    want = ref.compress(data, flags=2)
-    assert z.memory_compress(data, 2) == want
+    key = "mix24M_s123/gzip/b0"
+    assert cases.same_as_ref(key, z.memory_compress(data, 2))
     monkeypatch.setenv("ZULTRA_CUDA_BATCH_BLOCKS", "8")
     s = z.Stream(2)
     raw = data.tobytes()
@@ -161,11 +147,11 @@ def test_multi_device_public_api_and_cli_vs_compiled_reference(z, ref, monkeypat
         assert st in (z.ZULTRA_OK, z.ZULTRA_STREAM_END)
         got.append(b)
     s.end()
-    assert st == z.ZULTRA_STREAM_END and b"".join(got) == want
+    assert st == z.ZULTRA_STREAM_END and cases.same_as_ref(key, b"".join(got))
     src = tmp_path / "in.bin"
     src.write_bytes(raw)
     cli = os.path.join(ROOT, "zultra_b200", "zultra")
     env = dict(os.environ, ZULTRA_CUDA_TRACE="1")
     r = subprocess.run([cli, str(src), str(tmp_path / "out.gz")], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE, env=env, check=True)
-    assert (tmp_path / "out.gz").read_bytes() == want
+    assert cases.same_as_ref(key, (tmp_path / "out.gz").read_bytes())
     assert b"devices %d" % n in r.stderr, r.stderr[-400:]      # the CLI really spread the stream over all GPUs

@@ -1,6 +1,6 @@
 """GPU parity tests: the CUDA path, called through the C-ABI / libzultra API, against
-(1) the committed golden vectors produced by the reference, (2) the compiled reference under oracle/_ref when it
-travelled with the snapshot, (3) size-independent properties (inflate round trip, checksums) at larger sizes.
+(1) the committed golden vectors produced by the reference, (2) fingerprints of the reference's outputs on larger
+inputs (tests/golden/ref_golden.npz), (3) size-independent properties (inflate round trip, checksums) at larger sizes.
 Bit-exact everywhere: this path is integer/byte work."""
 import hashlib
 import os
@@ -11,7 +11,6 @@ import numpy as np
 import pytest
 
 import cases
-import refharness
 from zultra_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -74,20 +73,15 @@ def test_multi_block_vs_golden(z, idx):
     assert _inflate(out, 2) == data.tobytes()
 
 
-def test_stages_vs_compiled_reference(ctx, ref):
-    """Wider stage diff when oracle/_ref travelled: SA|LCP words, match lists, splits, code lengths, parse."""
-    rng = np.random.default_rng(5)
-    wins = [(synth.enwik(400000, seed=41), 32768), (synth.mozilla(500000, seed=42), 32768), (synth.mozilla(200000, seed=43), 1000),
-            (np.concatenate([np.zeros(70000, dtype=np.uint8), rng.integers(0, 4, size=50000).astype(np.uint8)]), 0)]
-    for win, hist in wins:
-        assert np.array_equal(ctx.window_sa_lcp(win), ref.sa_lcp(win))
-        assert np.array_equal(ctx.window_matches(win, hist), ref.matches(win, hist))
-        a, b = ctx.block_stages(win, hist), ref.block_stages(win, hist)
-        assert a["n"] == b["n"] and np.array_equal(a["info"][:, 1], b["split"])
-        assert np.array_equal(a["info"][:, 2], b["dyn"]) and np.array_equal(a["info"][:, 3], b["sc"]) and np.array_equal(a["info"][:, 4], b["dc"])
-        assert np.array_equal(a["ll"], b["ll"]) and np.array_equal(a["ol"], b["ol"])
-        assert np.array_equal(a["best"][hist:], b["best"][hist:])
-        assert np.array_equal(a["info"][:, 5], b["bits"])
+def test_stages_vs_compiled_reference(ctx):
+    """Wider stage diff against the reference's stage dumps: SA|LCP words, match lists, splits, static/dynamic decision
+    and costs, code lengths, parse, body bits."""
+    for i, (win, hist) in enumerate(cases.stage_windows()):
+        a = ctx.block_stages(win, hist)
+        got = dict(n=np.array([a["n"]]), split=a["info"][:, 1], dyn=a["info"][:, 2], sc=a["info"][:, 3], dc=a["info"][:, 4], ll=a["ll"], ol=a["ol"],
+                   best=a["best"][hist:], bits=a["info"][:, 5], sa_lcp=ctx.window_sa_lcp(win), match=ctx.window_matches(win, hist))
+        for k, v in got.items():
+            assert np.array_equal(cases.fingerprint(v), cases.ref_fp("stage%d/%s" % (i, k))), (i, hist, k)
 
 
 def test_streaming_api_equals_one_shot(z):
@@ -152,53 +146,34 @@ def test_large_roundtrip_properties(z):
     assert out[-8:-4] == zlib.crc32(raw).to_bytes(4, "little") and out[-4:] == (len(raw) & 0xffffffff).to_bytes(4, "little")
 
 
-def test_large_vs_compiled_reference(z, ref):
+def test_large_vs_compiled_reference(z):
     data = synth.mix(5 << 20, seed=100, seg_lo=300000, seg_hi=2 << 20)
     for flags in (0, 2):
-        assert z.memory_compress(data, flags) == ref.compress(data, flags=flags)
+        assert cases.same_as_ref("mix5M_s100/%s/b0" % cases.FMT[flags], z.memory_compress(data, flags)), flags
 
 
-def test_runs_and_periodic_vs_compiled_reference(z, ref):
+def test_runs_and_periodic_vs_compiled_reference(z):
     """Byte runs and long periodic repeats: the parse does not re-synchronise there, so these inputs go through the
     chain repair (zb_parse_fix_k), including its scan path for blocks made of literals and far leave-alone matches."""
-    rng = np.random.default_rng(17)
-    parts = []
-    for _ in range(60):
-        run = int(np.exp(rng.uniform(np.log(16), np.log(200000))))
-        parts.append(np.full(run, int(rng.choice([0, 0xFF, 0x41])), dtype=np.uint8))
-        parts.append(rng.integers(0, 256, size=int(rng.integers(1, 300))).astype(np.uint8))
-    rec = np.zeros((40000, 16), dtype=np.uint8)
-    rec[:, 0:4] = (np.arange(40000, dtype=np.uint32) + 77).astype("<u4").view(np.uint8).reshape(-1, 4)
-    rec[:, 8] = rng.integers(0, 4, size=40000)
-    parts.append(rec.reshape(-1))
-    parts.append(np.tile(rng.integers(0, 256, size=300).astype(np.uint8), 1500))
-    parts.append(np.tile(np.frombuffer(b"ab", dtype=np.uint8), 150000))
-    parts.append(synth.enwik(300000, seed=41))
-    parts.append(np.zeros(700000, dtype=np.uint8))
-    data = np.concatenate(parts)
+    data = cases.runs_and_periodic()
     for flags, block in ((0, 0), (2, 262144)):
-        assert z.memory_compress(data, flags, block) == ref.compress(data, flags=flags, block=block)
+        assert cases.same_as_ref("runs/%s/b%d" % (cases.FMT[flags], block), z.memory_compress(data, flags, block)), flags
 
 
-def test_lanes_vs_compiled_reference(z, ref, monkeypatch):
+def test_lanes_vs_compiled_reference(z, monkeypatch):
     """Block ranges of one call run as concurrent lanes (zb_capi.cu run_lanes); the stitched stream must equal the
     reference byte for byte, including stored sub-blocks whose size depends on the entering bit phase, a history that
     is not contiguous with the data, an entering bit count and the running checksum."""
-    rng = np.random.default_rng(5)
-    data = np.concatenate([synth.enwik(700000, seed=31), rng.integers(0, 256, size=300000).astype(np.uint8), synth.mozilla(900000, seed=32),
-                           rng.integers(0, 256, size=150000).astype(np.uint8), synth.enwik(450000, seed=33)])
+    data = cases.lanes_input()
     monkeypatch.setenv("ZULTRA_CUDA_LANE_MIN_BLOCKS", "1")
     for lanes, block in ((3, 262144), (4, 131072), (7, 65536)):
         monkeypatch.setenv("ZULTRA_CUDA_LANES", str(lanes))
         c = z.CudaCtx()
         try:
             for flags in (0, 1, 2):
-                want = ref.compress(data, flags=flags, block=block)
-                hdr = 0 if flags == 0 else (2 if flags == 1 else 10)
-                ftr = 0 if flags == 0 else (4 if flags == 1 else 8)
                 got, bits, ck = c.compress_blocks(data, block=block, finalize=1, flags=flags)
                 assert c.counters()["r5"] == lanes
-                assert got == want[hdr:len(want) - ftr], (lanes, block, flags)
+                assert cases.same_as_ref("lanes/%s/b%d/body" % (cases.FMT[flags], block), got), (lanes, block, flags)
                 if flags == 1:
                     assert ck == zlib.adler32(data.tobytes())
                 if flags == 2:
@@ -207,14 +182,13 @@ def test_lanes_vs_compiled_reference(z, ref, monkeypatch):
             cut = 4 * block
             a, abits, ack = c.compress_blocks(data[:cut], block=block, finalize=0, flags=2)
             b, bbits, bck = c.compress_blocks(data[cut:], hist=data[cut - 32768:cut].copy(), block=block, finalize=1, in_bits=abits & 7, flags=2, checksum=ack)
-            want = ref.compress(data, flags=2, block=block)[10:-8]
             joined = bytearray(a)
             if abits & 7:
                 joined[-1] |= b[0]
                 joined += b[1:]
             else:
                 joined += b
-            assert bytes(joined) == want and bck == zlib.crc32(data.tobytes())
+            assert cases.same_as_ref("lanes/gzip/b%d/body" % block, bytes(joined)) and bck == zlib.crc32(data.tobytes())
         finally:
             c.close()
 
@@ -231,11 +205,8 @@ def test_cli_drop_in(z, tmp_path):
         _gold("js48k/%s" % flag[1:], dst.read_bytes())
     assert subprocess.run([cli, "-d", str(src), str(tmp_path / "x")]).returncode == 100
     assert subprocess.run([cli, "-gzip", "-D", str(src), str(src), str(tmp_path / "x")], capture_output=True).returncode == 100
-    ref_cli = os.path.join(ROOT, "oracle", "_ref", "zultra_ref")
-    if os.path.exists(ref_cli):
-        big = tmp_path / "big.bin"
-        big.write_bytes(synth.mozilla(1500000, seed=13).tobytes())
-        subprocess.check_call([cli, str(big), str(tmp_path / "a.gz")], stdout=subprocess.DEVNULL)
-        subprocess.check_call([ref_cli, str(big), str(tmp_path / "b.gz")], stdout=subprocess.DEVNULL)
-        assert (tmp_path / "a.gz").read_bytes() == (tmp_path / "b.gz").read_bytes()
+    big = tmp_path / "big.bin"
+    big.write_bytes(synth.mozilla(1500000, seed=13).tobytes())
+    subprocess.check_call([cli, str(big), str(tmp_path / "a.gz")], stdout=subprocess.DEVNULL)
+    assert cases.same_as_ref("moz1.5M_s13/gzip/b0", (tmp_path / "a.gz").read_bytes())
     assert subprocess.run([cli, "-quicktest"], capture_output=True).returncode == 0
