@@ -272,10 +272,35 @@ inline void ZbPipe::setup(const std::vector<ZbWinDesc> &wins, const uint8_t *h_i
 
 /* ============================================================ suffix array + LCP ============================================================
  * Replaces divsufsort_build_array (divsufsort.c:377) and the PLCP/LCP/pack steps of matchfinder.c:57-90.
- * Prefix doubling: sort all suffixes of all windows by (window, first nb bytes), then repeatedly sort the
- * still-tied groups by the rank of the suffix h positions further on.  A suffix that runs off its window end
- * is smaller than any longer suffix it is a prefix of (no sentinel; the reference's order, SURVEY A-20).
+ * Prefix doubling: sort all suffixes of all windows by (window, first nb bytes), order every tied group of at most
+ * ZB_SA_LOCAL suffixes by its next 8 bytes in place (zb_sa_key), then repeatedly sort the still-tied groups by the rank of
+ * the suffix h positions further on.  A suffix that runs off its window end is smaller than any longer suffix it is a
+ * prefix of (no sentinel; the reference's order, SURVEY A-20).
  */
+#define ZB_SA_LOCAL 32    /* tied groups up to this size are ordered by their members' text, each member counting the ones before it */
+
+/* Order key of the suffix at window offset i (window of len bytes, text t) among suffixes that agree on their first d
+   bytes, zero-padded past the window end: the next 8 bytes big-endian, zero-padded (w), then min(suffix length, d + 9)
+   (tl).  A suffix ending inside the 8 bytes sorts before every longer one it is a prefix of, the shorter first; two
+   different suffixes of one window with equal keys both run on past d + 8 bytes and agree on all of them.  d >= 3. */
+ZB_HD void zb_sa_key(const uint8_t *t, uint32_t i, uint32_t len, uint32_t d, uint64_t &w, uint32_t &tl) {
+   const uint32_t rem = len - i;
+   tl = rem < d + 9 ? rem : d + 9;
+#ifdef __CUDA_ARCH__
+   if ((uint64_t)i + d + 12 <= len) {   /* three aligned words, all inside the window (d >= 3: none starts before the input) */
+      const uintptr_t a = (uintptr_t)(t + i + d);
+      const uint32_t *pa = (const uint32_t *)(a & ~(uintptr_t)3);
+      const uint32_t sh = (uint32_t)(a & 3) << 3;
+      const uint32_t x0 = __funnelshift_r(pa[0], pa[1], sh), x1 = __funnelshift_r(pa[1], pa[2], sh);
+      w = ((uint64_t)__byte_perm(x0, 0, 0x0123) << 32) | __byte_perm(x1, 0, 0x0123);
+      return;
+   }
+#endif
+   uint64_t x = 0;
+   for (uint32_t b = 0; b < 8; b++) x = (x << 8) | ((uint64_t)i + d + b < len ? t[i + d + b] : 0u);
+   w = x;
+}
+
 inline void ZbPipe::stage_sa() {
    const long n = P;
    keyA.need(n); keyB.need(n); valA.need(n); valB.need(n); rank.need(n); sa.need(n); actA.need(n); actB.need(n); tmpA.need(n + 1); tmpB.need(n + 1);
@@ -301,17 +326,42 @@ inline void ZbPipe::stage_sa() {
       vA[g] = (uint32_t)g;
    }, 256);
    zb_sort_pairs(st, keyA.p, valA.p, keyB.p, valB.p, n, 0, 8 * nbytes + wb, scratch.p);
-   /* initial groups */
+   /* initial groups.  Each suffix finds its group [gh, ge) in the sorted keys: a singleton is final; a member of a group of
+      at most ZB_SA_LOCAL counts the members whose key (zb_sa_key, 8 more bytes) is smaller, and the equal ones ahead of it,
+      which gives its slot and its rank (the slot of its first equal member); members of larger groups stay in place with
+      the group's first slot as rank.  head[j] = 1 marks slot j as still tied: all of a large group, members of a small one
+      with an equal key.  Every rank is the slot of the first suffix that agrees with it on at least nbytes bytes. */
    uint32_t *head = tmpA.p, *grp = tmpB.p, *rk = rank.p, *SA = sa.p, *act = actA.p, *act2 = actB.p, *cnt = counters.p;
-   zb_launch(st, n, ZB_LAMBDA(long j) { head[j] = (j == 0 || kA[j] != kA[j - 1]) ? (uint32_t)j : 0u; SA[j] = vA[j]; }, 256);
-   zb_inclusive_max(st, head, grp, n, scratch.p);
-   /* ranks, and active = members of groups with more than one suffix (one pass over grp for both) */
-   zb_launch(st, n, ZB_LAMBDA(long j) {
-      const uint32_t gj = grp[j];
-      rk[vA[j]] = gj;
-      bool is_head = gj == (uint32_t)j;
-      bool next_head = (j + 1 == n) || grp[j + 1] == (uint32_t)(j + 1);
-      head[j] = (is_head && next_head) ? 0u : 1u;
+   const int kbits = 8 * nbytes;
+   zb_tag("sa_group");
+   zb_launch(st, n, ZB_LAMBDA(long jl) {
+      const uint32_t j = (uint32_t)jl;
+      const uint64_t key = kA[j];
+      /* first member: gallop back, then bisect (lo < gh: kA[lo] differs or lo = -1) */
+      uint32_t gh = j, step = 1;
+      while (gh >= step && kA[gh - step] == key) { gh -= step; step <<= 1; }
+      long lo = gh >= step ? (long)(gh - step) : -1L;
+      while ((long)gh - lo > 1) { const uint32_t mid = (uint32_t)((lo + (long)gh) >> 1); if (kA[mid] == key) gh = mid; else lo = mid; }
+      const uint32_t g = vA[j];
+      if ((long)gh + ZB_SA_LOCAL < n && kA[gh + ZB_SA_LOCAL] == key) { SA[j] = g; rk[g] = gh; head[j] = 1u; return; }
+      uint32_t ge = j + 1;
+      while ((long)ge < n && kA[ge] == key) ge++;
+      if (ge - gh == 1) { SA[j] = g; rk[g] = j; head[j] = 0u; return; }
+      const int w = (int)(key >> kbits);
+      const uint32_t base = wbs[w], len = wd[w].len;
+      const uint8_t *t = T + wd[w].in_off;
+      uint64_t kw; uint32_t kt;
+      zb_sa_key(t, g - base, len, (uint32_t)nbytes, kw, kt);
+      uint32_t less = 0, eq_before = 0, eq = 0;
+      for (uint32_t y = gh; y < ge; y++) {
+         if (y == j) continue;
+         uint64_t yw; uint32_t yt;
+         zb_sa_key(t, vA[y] - base, len, (uint32_t)nbytes, yw, yt);
+         if (yw < kw || (yw == kw && yt < kt)) less++;
+         else if (yw == kw && yt == kt) { eq++; if (y < j) eq_before++; }
+      }
+      const uint32_t p = gh + less + eq_before;
+      SA[p] = g; rk[g] = gh + less; head[p] = eq ? 1u : 0u;
    }, 256);
    zb_exclusive_sum(st, head, grp, n, cnt, scratch.p);
    zb_launch(st, n, ZB_LAMBDA(long j) { if (head[j]) act[grp[j]] = (uint32_t)j; }, 256);
