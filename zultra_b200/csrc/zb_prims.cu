@@ -323,17 +323,23 @@ void zb_sort_pairs(zb_stream_t st, uint64_t *keys, uint32_t *vals, uint64_t *key
    (~1.08 M words) into its ~33 units of 32768 main + 32768 look-back positions - that was 26 words streamed per window position
    over two levels.  Every position belongs to at most TWO units (the one it is a main position of, and the next one, whose
    look-back it is in), so the cut is a stable partition: the window's list is read in segments of 4096 ranks, twice
-   (count, then scatter), and every entry is routed to its units.  Per segment and unit a 4096-bit membership bitmap in shared
-   memory gives an entry's rank among the unit's entries of the segment (popcounts) and its predecessor there (highest set bit
-   below); the LCP an entry gets in a unit's list is the minimum of the window LCPs after that predecessor up to itself
-   (32-entry block minima bound the scan of a long gap), and across segments the counts and the trailing minima are chained by a
-   small per-unit scan.  Same lists, bit for bit, as filtering the window list for every unit separately. */
+   (count, then scatter), and every entry is routed to its units.  The LCP an entry gets in a unit's list is the minimum of the
+   window LCPs after the unit's previous member up to the entry itself.  The count pass keeps per unit only its number of entries
+   (warp-aggregated shared counters), its last member (atomicMax) and the minimum LCP after that member; across segments these are
+   chained by a small per-unit scan.  The scatter pass keeps a 4096-bit membership bitmap per unit: popcounts give an entry's rank
+   among the unit's entries of the segment, the highest set bit below it in its 32-entry word its predecessor there.  A warp
+   handles exactly one such word (32 consecutive ranks) at a time and holds its LCPs in registers, so a gap minimum inside the
+   word is two shuffles of a sparse table over the lanes; a gap that starts in an earlier word is the minimum up to the word,
+   which a per-unit scan over the words computes once per segment (from in-block suffix minima and block minima, seeded with the
+   minimum carried in from earlier segments).  Same lists, bit for bit, as filtering the window list for every unit separately. */
 #define DS_SEG 4096
 #define DS_THREADS 256
 #define DS_WORDS (DS_SEG / 32)
 #define DS_BROW (DS_WORDS + 1)      /* bitmap row stride in words, prefix row stride in u16 pairs: rows of different units start in different banks
                                        (the lanes of a warp look at the SAME word index of DIFFERENT units: unpadded, a 32-way bank conflict per access) */
 #define DS_PROW (DS_WORDS + 2)
+#define DS_SROW 33                  /* suffix-minimum row stride in u16: the word scan reads a different block's row in every lane, and rows of 32 would put
+                                       every other lane in the same bank */
 
 __device__ __forceinline__ int ds_find_win(const ZbDistWin *dw, int nwin, uint32_t seg) {
    int lo = 0, hi = nwin - 1;
@@ -341,15 +347,30 @@ __device__ __forceinline__ int ds_find_win(const ZbDistWin *dw, int nwin, uint32
    return lo;
 }
 
+/* min(l[a .. lane]) over the lanes of a warp, a <= lane, where win[j] = min(l[lane - 2^j + 1 .. lane]) (cut at lane 0): the two
+   windows of length 2^j, j = floor(log2(lane - a + 1)), ending at lane and starting at a cover the range.  All lanes call it. */
+__device__ __forceinline__ uint32_t ds_lane_range_min(const uint32_t (&win)[6], int a, int lane) {
+   const int k = 31 - __clz(lane - a + 1);
+   uint32_t m = 0;
+#pragma unroll
+   for (int j = 0; j < 6; j++) {
+      const uint32_t o = __shfl_sync(0xffffffffu, win[j], (a + (1 << j) - 1) & 31);
+      if (j == k) m = min(win[j], o);
+   }
+   return m;
+}
+
 template <bool SCATTER>
 __global__ void __launch_bounds__(DS_THREADS) unit_dist_k(const uint32_t *sa_lcp, const ZbDistWin *dw, int nwin, int nu_max, uint32_t *segrec, uint32_t *unit_words) {
    extern __shared__ uint32_t ds_sm[];
-   uint32_t *bm = ds_sm;                                         /* [nu][DS_WORDS] membership bitmaps */
-   uint16_t *pre = (uint16_t *)(bm + (size_t)nu_max * DS_BROW); /* [nu][DS_WORDS] set bits before each word */
-   uint16_t *lcp = pre + (size_t)nu_max * DS_PROW;              /* [DS_SEG] */
-   uint16_t *bmin = lcp + DS_SEG;                                /* [DS_WORDS] minimum of every 32-entry block */
-   uint32_t *uoff = (uint32_t *)(bmin + DS_WORDS);               /* [nu + 1] SCATTER: where each unit's entries of this segment start in `stage` */
-   uint32_t *stage = uoff + nu_max + 1;                          /* [2 * DS_SEG] SCATTER: the segment's output, unit by unit, so that it leaves in runs */
+   uint16_t *smin = (uint16_t *)ds_sm;                           /* [DS_WORDS][DS_SROW] minimum of lcp[i .. end of i's block] */
+   uint16_t *bmin = smin + DS_WORDS * DS_SROW;                   /* [DS_WORDS] minimum of every 32-entry block */
+   uint32_t *ucnt = (uint32_t *)(bmin + DS_WORDS);               /* [nu + 1] entries per unit; SCATTER: turned into where each unit's entries start in `stage` */
+   int *ulast = (int *)(ucnt + nu_max + 1);                      /* [nu] count pass: rank of the unit's last member */
+   uint32_t *bm = (uint32_t *)(ulast + nu_max);                  /* [nu][DS_WORDS] SCATTER: membership bitmaps */
+   uint16_t *pre = (uint16_t *)(bm + (size_t)nu_max * DS_BROW);  /* [nu][DS_WORDS] SCATTER: members before each word */
+   uint16_t *gap = pre + (size_t)nu_max * DS_PROW;               /* [nu][DS_WORDS] SCATTER: minimum LCP after the last member before each word, up to the word */
+   uint32_t *stage = (uint32_t *)(gap + (size_t)nu_max * DS_PROW); /* [2 * DS_SEG] SCATTER: the segment's output, unit by unit, so that it leaves in runs */
    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
    const int w = ds_find_win(dw, nwin, blockIdx.x);
    const ZbDistWin W = dw[w];
@@ -376,104 +397,115 @@ __global__ void __launch_bounds__(DS_THREADS) unit_dist_k(const uint32_t *sa_lcp
       const uint32_t idx = (uint32_t)k * DS_THREADS + tid;
       wv[k] = idx < nr ? __ldg(sa_lcp + W.sa_base + r0 + idx) : (0x1ffu << ZB_POS_BITS);
    }
-   for (int e = tid; e < nu * DS_BROW; e += DS_THREADS) bm[e] = 0;
+   if (SCATTER) { for (int e = tid; e < nu * DS_BROW; e += DS_THREADS) bm[e] = 0; }
+   else { for (int u = tid; u < nu; u += DS_THREADS) { ucnt[u] = 0; ulast[u] = -1; } }
    __syncthreads();
+   /* entry idx = k * DS_THREADS + tid: warp `warp` holds block idx >> 5 whole, lane = idx & 31 */
 #pragma unroll
    for (int k = 0; k < DS_SEG / DS_THREADS; k++) {
       const uint32_t idx = (uint32_t)k * DS_THREADS + tid;
-      uint32_t v = wv[k];
-      if (idx < nr) {
-         const uint32_t p = v & ZB_POS_MASK;
-         const int ua = p < W.hist ? 0 : (int)((p - W.hist) >> 15);
-         atomicOr(bm + ua * DS_BROW + (idx >> 5), 1u << (idx & 31));
-         if (p >= W.hist && ua + 1 < nu) atomicOr(bm + (ua + 1) * DS_BROW + (idx >> 5), 1u << (idx & 31));
+      const uint32_t v = wv[k], p = v & ZB_POS_MASK;
+      const int ua = p < W.hist ? 0 : (int)((p - W.hist) >> 15);
+      const bool in = idx < nr, dual = p >= W.hist && ua + 1 < nu;
+      if (SCATTER) {
+         if (in) {
+            atomicOr(bm + ua * DS_BROW + (idx >> 5), 1u << lane);
+            if (dual) atomicOr(bm + (ua + 1) * DS_BROW + (idx >> 5), 1u << lane);
+         }
+      } else {
+#pragma unroll
+         for (int q = 0; q < 2; q++) {
+            const int u = in && (q == 0 || dual) ? ua + q : -1;
+            const uint32_t peers = __match_any_sync(0xffffffffu, (uint32_t)u);
+            if (u >= 0 && lane == 31 - __clz((int)peers)) { atomicAdd(ucnt + u, (uint32_t)__popc(peers)); atomicMax(ulast + u, (int)idx); }
+         }
       }
-      wv[k] = v;
-      lcp[idx] = (uint16_t)((v >> ZB_POS_BITS) & 0x1ffu);
-   }
-   __syncthreads();
-   /* block minima (one warp reduction per 32 entries) */
-   for (int b = warp; b < DS_WORDS; b += DS_THREADS / 32) {
-      const uint32_t m = __reduce_min_sync(0xffffffffu, (uint32_t)lcp[b * 32 + lane]);
-      if (lane == 0) bmin[b] = (uint16_t)m;
+      uint32_t s = (v >> ZB_POS_BITS) & 0x1ffu;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) { const uint32_t o = __shfl_down_sync(0xffffffffu, s, d); if (lane + d < 32) s = min(s, o); }
+      smin[(idx >> 5) * DS_SROW + lane] = (uint16_t)s;
+      if (lane == 0) bmin[idx >> 5] = (uint16_t)s;
    }
    __syncthreads();
    uint32_t *rec = segrec + (size_t)blockIdx.x * nu_max * 2;
    if (!SCATTER) {
       /* per unit: entries in this segment, and the minimum LCP after its last entry (over the whole segment if it has none) */
       for (int u = warp; u < nu; u += DS_THREADS / 32) {
-         const uint32_t *b = bm + u * DS_BROW;
-         uint32_t c = 0; int last = -1;
-#pragma unroll
-         for (int j = 0; j < DS_WORDS / 32; j++) {
-            const uint32_t x = b[j * 32 + lane];
-            c += (uint32_t)__popc(x);
-            if (x) last = (j * 32 + lane) * 32 + 31 - __clz((int)x);
-         }
-#pragma unroll
-         for (int d = 16; d > 0; d >>= 1) { c += __shfl_xor_sync(0xffffffffu, c, d); last = max(last, __shfl_xor_sync(0xffffffffu, last, d)); }
-         /* min of lcp[last + 1 .. nr): the rest of last's block, then whole blocks */
-         uint32_t m = 0x1ffu;
-         const int from = last + 1;
-         const int fb = (from + 31) >> 5;
-         { const int i = from + lane; if (i < fb * 32 && i < DS_SEG) m = lcp[i]; }
+         const int last = ulast[u], from = last + 1, fb = (from + 31) >> 5;
+         uint32_t m = lane == 0 && (from & 31) ? (uint32_t)smin[(from >> 5) * DS_SROW + (from & 31)] : 0x1ffu;
          for (int bb = fb + lane; bb < DS_WORDS; bb += 32) m = min(m, (uint32_t)bmin[bb]);
          m = __reduce_min_sync(0xffffffffu, m);
-         if (lane == 0) { rec[2 * u] = c; rec[2 * u + 1] = m | (last >= 0 ? 0x10000u : 0u); }
+         if (lane == 0) { rec[2 * u] = ucnt[u]; rec[2 * u + 1] = m | (last >= 0 ? 0x10000u : 0u); }
       }
       return;
    }
-   /* set bits before every bitmap word */
+   /* per unit and bitmap word: set bits before the word, and the minimum LCP from after the unit's last member before the word
+      (from the segment start, seeded with the minimum carried in, if there is none) up to the word's start.  A word with members
+      restarts that minimum at the LCPs after its last member, a word without continues it with its block minimum. */
    for (int u = warp; u < nu; u += DS_THREADS / 32) {
       const uint32_t *b = bm + u * DS_BROW;
-      uint32_t run = 0;
+      uint32_t run = 0, gin = rec[2 * u + 1];
 #pragma unroll
       for (int j = 0; j < DS_WORDS / 32; j++) {
-         const uint32_t c = (uint32_t)__popc(b[j * 32 + lane]);
+         const int wd = j * 32 + lane;
+         const uint32_t x = b[wd];
+         const uint32_t c = (uint32_t)__popc(x);
          uint32_t inc = c;
 #pragma unroll
          for (int d = 1; d < 32; d <<= 1) { const uint32_t o = __shfl_up_sync(0xffffffffu, inc, d); if (lane >= d) inc += o; }
-         pre[u * DS_PROW + j * 32 + lane] = (uint16_t)(run + inc - c);
+         pre[u * DS_PROW + wd] = (uint16_t)(run + inc - c);
          run += __shfl_sync(0xffffffffu, inc, 31);
+         const int t = 32 - __clz((int)x);      /* first offset after the word's last member */
+         uint32_t f = x != 0, g = x == 0 ? (uint32_t)bmin[wd] : t < 32 ? (uint32_t)smin[wd * DS_SROW + t] : 0x1ffu;
+#pragma unroll
+         for (int d = 1; d < 32; d <<= 1) {
+            const uint32_t fo = __shfl_up_sync(0xffffffffu, f, d), go = __shfl_up_sync(0xffffffffu, g, d);
+            if (lane >= d) { if (!f) g = min(g, go); f |= fo; }
+         }
+         const uint32_t incl = f ? g : min(gin, g);
+         const uint32_t excl = __shfl_up_sync(0xffffffffu, incl, 1);
+         gap[u * DS_PROW + wd] = (uint16_t)(lane == 0 ? gin : excl);
+         gin = __shfl_sync(0xffffffffu, incl, 31);
       }
-      if (lane == 0) uoff[u + 1] = run;      /* the unit's count, turned into a start below */
+      if (lane == 0) ucnt[u + 1] = run;      /* the unit's count, turned into a start below */
    }
    __syncthreads();
-   if (tid == 0) { uint32_t acc = 0; uoff[0] = 0; for (int u = 0; u < nu; u++) { const uint32_t c = uoff[u + 1]; uoff[u + 1] = acc + c; acc += c; } }
+   if (tid == 0) { uint32_t acc = 0; ucnt[0] = 0; for (int u = 0; u < nu; u++) { const uint32_t c = ucnt[u + 1]; ucnt[u + 1] = acc + c; acc += c; } }
    __syncthreads();
 #pragma unroll
    for (int k = 0; k < DS_SEG / DS_THREADS; k++) {
-      const uint32_t idx = (uint32_t)k * DS_THREADS + tid;
-      if (idx >= nr) continue;
-      const uint32_t p = wv[k] & ZB_POS_MASK;
+      const uint32_t idx = (uint32_t)k * DS_THREADS + tid, wi = idx >> 5;
+      const uint32_t v = wv[k], p = v & ZB_POS_MASK;
       const int ua = p < W.hist ? 0 : (int)((p - W.hist) >> 15);
-      const int nun = (p >= W.hist && ua + 1 < nu) ? 2 : 1;
-      for (int q = 0; q < nun; q++) {
+      const bool in = idx < nr, dual = p >= W.hist && ua + 1 < nu;
+      uint32_t win[6];
+      win[0] = (v >> ZB_POS_BITS) & 0x1ffu;
+#pragma unroll
+      for (int j = 1; j < 6; j++) { const uint32_t o = __shfl_up_sync(0xffffffffu, win[j - 1], 1 << (j - 1)); win[j] = lane >= (1 << (j - 1)) ? min(win[j - 1], o) : win[j - 1]; }
+#pragma unroll
+      for (int q = 0; q < 2; q++) {
+         const bool on = in && (q == 0 || dual);
          const int u = ua + q;
-         const uint32_t *b = bm + u * DS_BROW;
-         const uint32_t wi = idx >> 5, below = b[wi] & ((1u << (idx & 31)) - 1u);
-         const uint32_t rank = (uint32_t)pre[u * DS_PROW + wi] + (uint32_t)__popc(below);
-         int prev = -1;
-         if (below) prev = (int)(wi * 32) + 31 - __clz((int)below);
-         else for (int x = (int)wi - 1; x >= 0; x--) { const uint32_t y = b[x]; if (y) { prev = x * 32 + 31 - __clz((int)y); break; } }
-         /* minimum of lcp[prev + 1 .. idx] */
-         uint32_t m = 0x1ffu;
-         const int from = prev + 1, fb = (from + 31) >> 5, lb = (int)(idx >> 5);
-         if (fb > lb) { for (int i = from; i <= (int)idx; i++) m = min(m, (uint32_t)lcp[i]); }
-         else {
-            for (int i = from; i < fb * 32; i++) m = min(m, (uint32_t)lcp[i]);
-            for (int bb = fb; bb < lb; bb++) m = min(m, (uint32_t)bmin[bb]);
-            for (int i = lb * 32; i <= (int)idx; i++) m = min(m, (uint32_t)lcp[i]);
+         uint32_t rank = 0, g = 0x1ffu;
+         int a = lane;
+         if (on) {
+            const uint32_t below = bm[u * DS_BROW + wi] & ((1u << lane) - 1u);
+            rank = (uint32_t)pre[u * DS_PROW + wi] + (uint32_t)__popc(below);
+            /* minimum of lcp[prev + 1 .. idx]: inside the word after a predecessor there, else from the word's start on top of the gap before it */
+            if (below) a = 32 - __clz((int)below);
+            else { a = 0; g = gap[u * DS_PROW + wi]; }
          }
-         if (prev < 0) m = min(m, rec[2 * u + 1]);      /* carried in from the segments before */
-         /* unit u of this window: main positions from hist + u * 32768, look-back 32768 before them */
-         const uint32_t m0 = W.hist + (uint32_t)u * ZB_MAX_OFFSET, ulo = m0 > ZB_MAX_OFFSET ? m0 - ZB_MAX_OFFSET : 0;
-         stage[uoff[u] + rank] = (p - ulo) | (m << ZB_POS_BITS);
+         const uint32_t m = min(g, ds_lane_range_min(win, a, lane));
+         if (on) {
+            /* unit u of this window: main positions from hist + u * 32768, look-back 32768 before them */
+            const uint32_t m0 = W.hist + (uint32_t)u * ZB_MAX_OFFSET, ulo = m0 > ZB_MAX_OFFSET ? m0 - ZB_MAX_OFFSET : 0;
+            stage[ucnt[u] + rank] = (p - ulo) | (m << ZB_POS_BITS);
+         }
       }
    }
    __syncthreads();
    for (int u = warp; u < nu; u += DS_THREADS / 32) {      /* a unit's entries of this segment are one run of its list */
-      const uint32_t a = uoff[u], n = uoff[u + 1] - a;
+      const uint32_t a = ucnt[u], n = ucnt[u + 1] - a;
       uint32_t *dst = unit_words + (size_t)(W.unit_base + u) * (2 * ZB_MAX_OFFSET) + rec[2 * u];
       for (uint32_t j = lane; j < n; j += 32) dst[j] = stage[a + j];
    }
@@ -503,11 +535,12 @@ __global__ void unit_dist_offsets_k(const ZbDistWin *dw, int nwin, int nu_max, u
 void zb_unit_distribute(zb_stream_t st, const uint32_t *sa_lcp, const ZbDistWin *dw, int nwin, int nseg_total, int total_units, int nu_max, uint32_t *segrec,
                         uint32_t *unit_words, uint32_t *unit_cnt) {
    if (nseg_total <= 0 || total_units <= 0) return;
-   const size_t smem = (size_t)nu_max * DS_BROW * 4 + (size_t)nu_max * DS_PROW * 2 + DS_SEG * 2 + DS_WORDS * 2 + ((size_t)nu_max + 1) * 4 + 2 * DS_SEG * 4 + 16;
-   ZB_CUDA_CHECK(cudaFuncSetAttribute(unit_dist_k<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
-   ZB_CUDA_CHECK(cudaFuncSetAttribute(unit_dist_k<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
+   const size_t smem_count = (size_t)DS_WORDS * DS_SROW * 2 + DS_WORDS * 2 + ((size_t)nu_max + 1) * 4 + (size_t)nu_max * 4;
+   const size_t smem = smem_count + (size_t)nu_max * DS_BROW * 4 + (size_t)nu_max * DS_PROW * 2 * 2 + 2 * DS_SEG * 4;
+   ZB_CUDA_CHECK(cudaFuncSetAttribute(unit_dist_k<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_count));
+   ZB_CUDA_CHECK(cudaFuncSetAttribute(unit_dist_k<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
    PROF_K("mf_unit_dist", st);
-   unit_dist_k<false><<<nseg_total, DS_THREADS, smem - 2 * DS_SEG * 4, st>>>(sa_lcp, dw, nwin, nu_max, segrec, unit_words);      /* the count pass has no staging area: twice the CTAs per SM */
+   unit_dist_k<false><<<nseg_total, DS_THREADS, smem_count, st>>>(sa_lcp, dw, nwin, nu_max, segrec, unit_words);      /* the count pass has no bitmaps and no staging area */
    unit_dist_offsets_k<<<(total_units + 127) / 128, 128, 0, st>>>(dw, nwin, nu_max, segrec, unit_cnt, total_units);
    unit_dist_k<true><<<nseg_total, DS_THREADS, smem, st>>>(sa_lcp, dw, nwin, nu_max, segrec, unit_words);
    PROF_E(st);
