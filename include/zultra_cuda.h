@@ -117,7 +117,8 @@ int zultra_cuda_block_stages(zultra_cuda_ctx_t *pCtx, const unsigned char *pWind
 
 /* milliseconds spent per stage in the last compress call: {h2d, sa+lcp, match, greedy+split, parse, emit, d2h, total} */
 int zultra_cuda_last_timings(zultra_cuda_ctx_t *pCtx, float *pMs8);
-/* counters of the last call: {windows, sub-blocks, suffix-sort rounds, parse chunks redone, kernel launches, stored sub-blocks, ub_hits, tiles} */
+/* counters of the last call: {windows, sub-blocks, suffix-sort rounds, parse chunks redone, kernel launches, 0 (unused),
+   devices of the last call spread over several devices (0 before the first), match-finder tiles} */
 int zultra_cuda_last_counters(zultra_cuda_ctx_t *pCtx, long long *pCounters8);
 
 /* kernels this library has launched in this process so far (all contexts, all host threads) */

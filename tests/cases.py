@@ -86,7 +86,7 @@ def parse_chunk_input(cd):
     return synth.mix(6 << 20, seed=300 + cd, seg_lo=400000, seg_hi=2 << 20)
 
 
-PARSE_CHUNKS = [(704, 1), (960, 1), (1856, 1), (2048, 1), (64, 1), (128, 1), (200, 1), (320, 1), (512, 0), (128, 0)]
+PARSE_CHUNKS = [704, 960, 1856, 2048, 64, 128, 200, 320, 512]
 
 
 def stage_windows():
@@ -121,7 +121,7 @@ def ref_streams():
             add("lanes", lanes_input, flags, block, "body")
     for flags in (0, 1, 2):
         add("oneshot10M", one_shot_320_blocks, flags, 32768)
-    for cd in sorted({cd for cd, _ in PARSE_CHUNKS}):
+    for cd in sorted(PARSE_CHUNKS):
         add("parse_chunk_cd%d" % cd, lambda cd=cd: parse_chunk_input(cd), 2, 0, "body")
     add("mix10M_s77", lambda: synth.mix(10 << 20, seed=77, seg_lo=1 << 20, seg_hi=3 << 20), 0)
     for seed, block in ((73, 131072), (74, 65536), (75, 262144)):

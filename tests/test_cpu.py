@@ -173,17 +173,16 @@ def test_emulated_compact_candidate_records_multi_block(emu, monkeypatch):
         assert cases.same_as_ref("%s/deflate/b%d" % (name, block), out), name
 
 
-@pytest.mark.parametrize("cd,awu,lean", [(64, "1", "0"), (320, "1", "1"), (128, "0", "0")])
-def test_emulated_adaptive_warmup_vs_golden(emu, monkeypatch, cd, awu, lean):
+@pytest.mark.parametrize("cd,lean", [(64, "0"), (320, "1"), (128, "0")])
+def test_emulated_adaptive_warmup_vs_golden(emu, monkeypatch, cd, lean):
     """Adaptive warm-up of the chunked parse (zb_pipeline.h stage_parse, D2): a chunk is verified over, and warmed up above,
     only the costs its own candidates reach (need(c) = max(reach(c), need(c - 1) - CD) for chunks shorter than the 258-position
-    horizon).  Host build, chunk lengths below, at and above the horizon, with the rule on and off, both recurrence forms:
-    same stream as the golden vectors, on text, binaries, byte runs and short-period data."""
+    horizon).  Host build, chunk lengths below, at and above the horizon, both recurrence forms: same stream as the golden
+    vectors, on text, binaries, byte runs and short-period data."""
     monkeypatch.setenv("ZB_EMU_PARSE_CD", str(cd))
-    monkeypatch.setenv("ZULTRA_CUDA_PARSE_AWU", awu)
     if lean == "1":
         monkeypatch.setenv("ZB_EMU_DP_LEAN", "1")
     for name in ("js48k", "moz300k", "enwik200k", "rows1000") + (("period7",) if cd >= 320 else ()):      # (the host repair loop is slow on short-period data with short chunks)
         data = cases.small_cases()[name]
         out, bits, _ = emu.compress(data)
-        assert _gold_ok("%s/deflate" % name, out), (name, cd, awu, lean)
+        assert _gold_ok("%s/deflate" % name, out), (name, cd, lean)

@@ -160,20 +160,17 @@ def test_runs_and_periodic_vs_compiled_reference(z):
         assert cases.same_as_ref("runs/%s/b%d" % (cases.FMT[flags], block), z.memory_compress(data, flags, block)), flags
 
 
-def test_lanes_vs_compiled_reference(z, monkeypatch):
-    """Block ranges of one call run as concurrent lanes (zb_capi.cu run_lanes); the stitched stream must equal the
-    reference byte for byte, including stored sub-blocks whose size depends on the entering bit phase, a history that
-    is not contiguous with the data, an entering bit count and the running checksum."""
+def test_compress_blocks_vs_compiled_reference(z):
+    """Several max-blocks in one zultra_cuda_compress_blocks call: the stream must equal the reference byte for byte,
+    including stored sub-blocks whose size depends on the entering bit phase, a history that is not contiguous with the
+    data, an entering bit count and the running checksum."""
     data = cases.lanes_input()
-    monkeypatch.setenv("ZULTRA_CUDA_LANE_MIN_BLOCKS", "1")
-    for lanes, block in ((3, 262144), (4, 131072), (7, 65536)):
-        monkeypatch.setenv("ZULTRA_CUDA_LANES", str(lanes))
+    for block in (262144, 131072, 65536):
         c = z.CudaCtx()
         try:
             for flags in (0, 1, 2):
                 got, bits, ck = c.compress_blocks(data, block=block, finalize=1, flags=flags)
-                assert c.counters()["r5"] == lanes
-                assert cases.same_as_ref("lanes/%s/b%d/body" % (cases.FMT[flags], block), got), (lanes, block, flags)
+                assert cases.same_as_ref("lanes/%s/b%d/body" % (cases.FMT[flags], block), got), (block, flags)
                 if flags == 1:
                     assert ck == zlib.adler32(data.tobytes())
                 if flags == 2:

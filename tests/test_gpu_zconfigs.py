@@ -121,21 +121,24 @@ def test_one_shot_across_256_block_batches_vs_compiled_reference(z):
         assert cases.same_as_ref("oneshot10M/%s/b32768" % cases.FMT[flags], z.memory_compress(data, flags, 32768)), flags
 
 
-@pytest.mark.parametrize("cd,awu", cases.PARSE_CHUNKS)
-def test_forced_parse_chunk_vs_compiled_reference(z, monkeypatch, cd, awu):
+@pytest.mark.parametrize("cd,name", [(cd, "mix6M") for cd in cases.PARSE_CHUNKS] + [(128, "mixed91"), (512, "mixed91")])
+def test_forced_parse_chunk_vs_compiled_reference(z, monkeypatch, cd, name):
     """The parse chunk length is chosen from the batch size (960 at 100 MB, up to 1856 for 256-block batches, 128 for small
-    inputs): force the lengths the configurations use on an input the reference finishes in seconds - with the adaptive
-    warm-up (a chunk's warm-up and the verified part of its signature follow what its candidates reach; chunks shorter than
-    the 258-position horizon take the propagated form need(c) = max(reach(c), need(c - 1) - CD)) and with it switched off."""
+    inputs): force the lengths the configurations use on an input the reference finishes in seconds.  The adaptive warm-up
+    follows what a chunk's candidates reach (its warm-up and the verified part of its signature); chunks shorter than the
+    258-position horizon take the propagated form need(c) = max(reach(c), need(c - 1) - CD).  Two lengths also run over
+    64 KiB max-blocks of the mixed stream, whose zero run and random stretches go through the repair chains."""
     monkeypatch.setenv("ZULTRA_CUDA_PARSE_CD", str(cd))
-    monkeypatch.setenv("ZULTRA_CUDA_PARSE_AWU", str(awu))
-    data = cases.parse_chunk_input(cd)
+    if name == "mixed91":
+        data, block, key = cases.mixed(91), 65536, "mixed91/gzip/b65536/body"
+    else:
+        data, block, key = cases.parse_chunk_input(cd), 0, "parse_chunk_cd%d/gzip/b0/body" % cd
     c = z.CudaCtx()
     try:
-        got, bits, ck = c.compress_blocks(data, finalize=1, flags=2)
+        got, bits, ck = c.compress_blocks(data, block=block, finalize=1, flags=2)
     finally:
         c.close()
-    assert cases.same_as_ref("parse_chunk_cd%d/gzip/b0/body" % cd, got) and ck == zlib.crc32(data.tobytes())
+    assert cases.same_as_ref(key, got) and ck == zlib.crc32(data.tobytes())
 
 
 def test_multi_wave_tile_lists_vs_compiled_reference(z, monkeypatch):

@@ -270,17 +270,14 @@ int main(int argc, char **argv) {
       if (dict && (opt & FMT_MASK) != FMT_ZLIB) { fprintf(stderr, "dictionaries are only supported for the zlib framing\n"); return 100; }
       r = do_compress(in, out, dict, opt);
       if (r == 0 && verify) r = do_compare(out, in, dict, opt);
-      /* all files are closed.  ZULTRA_CLI_EXIT: 0 = plain return, 1 = _exit without the CUDA runtime's exit handlers (default),
-         2 = free the pooled contexts first; with ZULTRA_CUDA_TRACE the milestones are printed so that the teardown can be timed */
+      /* all files are closed: _exit without the CUDA runtime's exit handlers; with ZULTRA_CUDA_TRACE the milestone is printed
+         so that the teardown can be timed */
       {
-         const char *e = getenv("ZULTRA_CLI_EXIT"), *tr = getenv("ZULTRA_CUDA_TRACE");
-         const int mode = e ? atoi(e) : 1;
-         if (tr && atoi(tr)) fprintf(stderr, "[cli %9.2f ms] streams closed, exit mode %d\n", (double)(now_us() - g_t0) / 1000.0, mode);
-         if (mode == 2) { zultra_cuda_release_cached(); if (tr && atoi(tr)) fprintf(stderr, "[cli %9.2f ms] contexts released\n", (double)(now_us() - g_t0) / 1000.0); }
+         const char *tr = getenv("ZULTRA_CUDA_TRACE");
+         if (tr && atoi(tr)) fprintf(stderr, "[cli %9.2f ms] streams closed\n", (double)(now_us() - g_t0) / 1000.0);
          fflush(NULL);
-         if (mode == 1) _exit(r);
+         _exit(r);
       }
-      return r;
    }
    if (cmd == 'B') return do_cbench(in, out, opt);
    return 100;

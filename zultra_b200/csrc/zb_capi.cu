@@ -16,11 +16,6 @@ struct zultra_cuda_ctx_s {
    float ms[8];
    long long counters[8];
    std::vector<uint8_t> out;
-   /* lanes: block ranges of one call run concurrently, each on its own stream / pipeline / host thread, so that the
-      latency-bound stages of one range overlap the issue-bound stages of another (see run_lanes) */
-   int nlanes = 1, lane_min_blocks = 4;   /* measured on B200: lanes do not pay (the big kernels are shared-memory / issue limited), kept for H2D overlap experiments */
-   std::vector<zultra_cuda_ctx_s *> lanes;
-   ZbBuf<uint32_t> lane_out;
    /* several devices behind one context (zultra_cuda_ctx_set_devices): peers[k - 1] is the context on device (device + k) % count */
    int ndev = 1;
    std::vector<zultra_cuda_ctx_s *> peers;
@@ -83,16 +78,10 @@ int zultra_cuda_ctx_create(zultra_cuda_ctx_t **pp, int device) {
    memset(c->ms, 0, sizeof(c->ms)); memset(c->counters, 0, sizeof(c->counters));
    if (cudaStreamCreateWithFlags(&c->pipe.st, cudaStreamNonBlocking) != cudaSuccess) { delete c; return ZULTRA_CUDA_ERR_CUDA; }
    zb_trace("ctx_create: stream created (primary context up)");
-   {  /* tuning knobs (never change the output) */
+   {  /* test hooks: chunk and tile lengths of large inputs on small ones (never change the output) */
       const char *e;
       if ((e = getenv("ZULTRA_CUDA_PARSE_CD")) && atoi(e) >= 64) c->pipe.parse_cd = atoi(e);
-      if ((e = getenv("ZULTRA_CUDA_PARSE_WU")) && atoi(e) >= 258) c->pipe.parse_wu = atoi(e);
       if ((e = getenv("ZULTRA_CUDA_TILE")) && atoi(e) >= 256) c->tile = (unsigned)atoi(e);
-      if ((e = getenv("ZULTRA_CUDA_EXACT_SA")) && atoi(e) > 0) c->pipe.sa_exact = true;
-      if ((e = getenv("ZULTRA_CUDA_TS_MIN")) && atoi(e) >= 1) c->pipe.mf_ts_min = atoi(e);
-      if ((e = getenv("ZULTRA_CUDA_TS_MUL")) && atoi(e) >= 0) c->pipe.mf_ts_mul = atoi(e);
-      if ((e = getenv("ZULTRA_CUDA_LANES")) && atoi(e) >= 1 && atoi(e) <= 16) c->nlanes = atoi(e);
-      if ((e = getenv("ZULTRA_CUDA_LANE_MIN_BLOCKS")) && atoi(e) >= 1) c->lane_min_blocks = atoi(e);
    }
    *pp = c;
    return 0;
@@ -101,10 +90,8 @@ int zultra_cuda_ctx_create(zultra_cuda_ctx_t **pp, int device) {
 void zultra_cuda_ctx_destroy(zultra_cuda_ctx_t *c) {
    if (!c) return;
    cudaSetDevice(c->device);
-   for (size_t i = 0; i < c->lanes.size(); i++) zultra_cuda_ctx_destroy(c->lanes[i]);
    for (size_t i = 0; i < c->peers.size(); i++) zultra_cuda_ctx_destroy(c->peers[i]);
    cudaSetDevice(c->device);
-   c->lane_out.release();
    c->pipe.release_all();
    cudaStreamDestroy(c->pipe.st);
    delete c;
@@ -130,122 +117,6 @@ static int run_one(zultra_cuda_ctx_t *c, const ZbStreamIn &s, unsigned block, Zb
    return rc;
 }
 
-/*
- * One call = consecutive max-blocks of one stream.  With enough blocks the range is cut into `nl` lanes of whole blocks;
- * each lane is a shard in the sense of zultra_cuda_shard_prepare (its own 32 KiB of preceding input as history) driven by
- * its own host thread on its own stream.  Everything up to the sub-block sizes is independent of the bit phase; the 8-entry
- * phase maps compose left to right into every lane's absolute bit offset (the same algebra as the multi-GPU stitch),
- * then all lanes emit into ONE zeroed word buffer, edge words merged with atomicOr.
- *   host_in != 0: [host_hist (hist_size) | host_in (n)] in host memory;  dev_in != 0: the same layout in device memory.
- */
-static int lanes_wanted(zultra_cuda_ctx_t *c, size_t n, unsigned block) {
-   const size_t nblocks = (n + block - 1) / block;
-   int nl = c->nlanes;
-   while (nl > 1 && nblocks < (size_t)nl * c->lane_min_blocks) nl--;
-   return nl;
-}
-
-static int run_lanes(zultra_cuda_ctx_t *c, int nl, const uint8_t *host_hist, int hist_size, const uint8_t *host_in, const uint8_t *dev_in, size_t n,
-                     unsigned block, int finalize, unsigned in_bits, unsigned flags, unsigned *checksum, uint8_t *host_out, uint8_t *dev_out, size_t out_cap,
-                     unsigned long long *out_bits) {
-   const long long l0 = g_zb_launches;
-   const size_t nblocks = (n + block - 1) / block, per = (nblocks + nl - 1) / nl;
-   while ((int)c->lanes.size() < nl) {
-      zultra_cuda_ctx_t *q = 0;
-      if (zultra_cuda_ctx_create(&q, c->device)) return ZULTRA_CUDA_ERR_CUDA;
-      c->lanes.push_back(q);
-   }
-   const int kind = (flags & 2) ? 2 : ((flags & 1) ? 1 : 0);
-   struct Lane { size_t lo, hi; int rc; ZbRunOpts o; unsigned ck; unsigned long long abs_bits, end_bits; };
-   std::vector<Lane> L(nl);
-   ZbTimer tot;
-   for (int k = 0; k < nl; k++) {
-      L[k].lo = std::min(n, (size_t)k * per * block); L[k].hi = std::min(n, (size_t)(k + 1) * per * block); L[k].rc = 0;
-      L[k].ck = k == 0 ? (checksum ? *checksum : 0) : (kind == 1 ? 1u : 0u);
-   }
-   auto prepare = [&](int k) {
-      zultra_cuda_ctx_t *q = k == 0 ? c : c->lanes[k];
-      Lane &l = L[k];
-      if (l.hi <= l.lo) return;
-      if (k) g_zb_cuda_error = 0;      /* the error flag is per host thread: a lane's failure comes back through l.rc */
-      cudaSetDevice(c->device);
-      const uint32_t h = k == 0 ? (uint32_t)hist_size : (uint32_t)ZB_HISTORY;
-      ZbStreamIn s;
-      if (dev_in) { ZbStreamIn t = {0, l.hi - l.lo, 0, h, (finalize && l.hi == n) ? 1 : 0, 0, l.ck}; s = t; l.o.dev_in = dev_in + hist_size + l.lo - h; }
-      else { ZbStreamIn t = {host_in + l.lo, l.hi - l.lo, k == 0 ? host_hist : host_in + l.lo - h, h, (finalize && l.hi == n) ? 1 : 0, 0, l.ck}; s = t; }
-      l.o.phase = 1; l.o.checksum_kind = kind; l.o.tile_main = c->tile;
-      q->pipe.parse_cd = c->pipe.parse_cd; q->pipe.parse_wu = c->pipe.parse_wu; q->pipe.mf_ts_min = c->pipe.mf_ts_min; q->pipe.mf_ts_mul = c->pipe.mf_ts_mul;
-      q->pipe.counters.need(64);
-      zb_memset(q->pipe.st, q->pipe.counters.p, 0, 64 * 4);
-      q->pipe.stat_redo = 0;
-      std::vector<ZbStreamRes> res;
-      l.rc = zb_run_batch(q->pipe, &s, 1, block, q->out, res, l.o);
-      if (zb_failed()) l.rc = -3;
-      if (l.rc == 0) l.ck = res[0].checksum;
-   };
-   {
-      std::vector<std::thread> th;
-      for (int k = 1; k < nl; k++) th.emplace_back(prepare, k);
-      prepare(0);
-      for (size_t i = 0; i < th.size(); i++) th[i].join();
-   }
-   if (getenv("ZULTRA_CUDA_LANE_TRACE")) {
-      double t0 = 1e300; for (int k = 0; k < nl; k++) t0 = std::min(t0, L[k].o.t_abs[0]);
-      for (int k = 0; k < nl; k++) fprintf(stderr, "lane %d: setup %.1f sa %.1f match %.1f split %.1f parse %.1f prep %.1f\n", k, L[k].o.t_abs[0] - t0, L[k].o.t_abs[1] - t0, L[k].o.t_abs[2] - t0, L[k].o.t_abs[3] - t0, L[k].o.t_abs[4] - t0, L[k].o.t_abs[5] - t0);
-   }
-   for (int k = 0; k < nl; k++) if (L[k].rc) return ZULTRA_CUDA_ERR_CUDA;
-   /* phase maps -> absolute bit offsets (tests/test_cpu_shards.py checks this algebra against the reference) */
-   unsigned long long pos = in_bits;
-   for (int k = 0; k < nl; k++) {
-      L[k].abs_bits = pos;
-      if (L[k].hi > L[k].lo) pos += L[k].o.phase_bits[pos & 7] - (pos & 7);
-   }
-   const size_t nb = (size_t)((pos + 7) / 8);
-   if (nb > out_cap) return ZULTRA_CUDA_ERR_DST;
-   const size_t nwords = (size_t)((pos + 31) / 32) + 4;
-   c->lane_out.need(nwords);
-   if (!c->lane_out.p) return ZULTRA_CUDA_ERR_CUDA;
-   zb_memset(c->pipe.st, c->lane_out.p, 0, nwords * 4);
-   zb_sync(c->pipe.st);
-   float t_prep = tot.lap();
-   auto emit = [&](int k) {
-      zultra_cuda_ctx_t *q = k == 0 ? c : c->lanes[k];
-      if (L[k].hi <= L[k].lo) return;
-      if (k) g_zb_cuda_error = 0;
-      cudaSetDevice(c->device);
-      L[k].rc = zb_finish_lane(q->pipe, L[k].abs_bits, c->lane_out.p, &L[k].end_bits);
-      if (zb_failed()) L[k].rc = -3;
-   };
-   {
-      std::vector<std::thread> th;
-      for (int k = 1; k < nl; k++) th.emplace_back(emit, k);
-      emit(0);
-      for (size_t i = 0; i < th.size(); i++) th[i].join();
-   }
-   for (int k = 0; k < nl; k++) if (L[k].rc) return ZULTRA_CUDA_ERR_CUDA;
-   if (dev_out) zb_d2d(c->pipe.st, dev_out, c->lane_out.p, nb);
-   else zb_d2h(c->pipe.st, host_out, c->lane_out.p, nb);
-   zb_sync(c->pipe.st);
-   *out_bits = pos;
-   if (checksum) {
-      unsigned ck = L[0].ck;
-      for (int k = 1; k < nl; k++) if (L[k].hi > L[k].lo) ck = zultra_cuda_checksum_combine(flags, ck, L[k].ck, L[k].hi - L[k].lo);
-      *checksum = ck;
-   }
-   /* stage times: the slowest lane per stage (they run side by side); counters: sums */
-   memset(c->ms, 0, sizeof(c->ms)); memset(c->counters, 0, sizeof(c->counters));
-   for (int k = 0; k < nl; k++) {
-      if (L[k].hi <= L[k].lo) continue;
-      ZbPipe &p = (k == 0 ? c : c->lanes[k])->pipe;
-      for (int i = 0; i < 7; i++) c->ms[i] = std::max(c->ms[i], L[k].o.ms[i]);
-      c->counters[0] += p.nwin; c->counters[1] += p.nsub; c->counters[2] = std::max<long long>(c->counters[2], p.stat_sa_rounds);
-      c->counters[3] += p.stat_redo; c->counters[7] += p.stat_tiles;
-   }
-   c->ms[5] += tot.lap(); c->ms[7] = t_prep + c->ms[5];
-   c->counters[4] = g_zb_launches - l0; c->counters[5] = nl;
-   return 0;
-}
-
 /* ============================================================ several GPUs behind one call ============================================================
  * A call = consecutive max-blocks of one stream (host memory in, host memory out).  The range is cut into CHUNKS of a few
  * max-blocks, dealt round-robin to the devices: every device gets a sample of the whole range, so a stream whose cost per
@@ -256,7 +127,7 @@ static int run_lanes(zultra_cuda_ctx_t *c, int nl, const uint8_t *host_hist, int
  *   1. DMA of every chunk [history | bytes] straight from the caller's buffer, pipeline up to the sub-block sizes,
  *      an 8-entry phase map and a checksum per chunk;
  *   2. (host) the maps compose left to right into every chunk's entering phase and absolute bit offset - the bit-offset
- *      scan of the stitch (same algebra as run_lanes; tests/test_cpu_shards.py checks it against the reference);
+ *      scan of the stitch (tests/test_cpu_shards.py checks this algebra against the reference);
  *   3. emission for the true phases, then every chunk's bytes go by DMA from its device straight to their byte offset in
  *      the caller's output buffer; the byte a chunk shares with its predecessor is OR-merged on the host.
  * No device-to-device traffic at all: the shard bitstreams meet in host memory, where the caller wants them.
@@ -268,15 +139,13 @@ static zultra_cuda_ctx_t *multi_dev_ctx(zultra_cuda_ctx_t *c, int k) {
       zultra_cuda_ctx_t *q = 0;
       const int dev = (c->device + (int)c->peers.size() + 1) % count;
       if (zultra_cuda_ctx_create(&q, dev)) return 0;
-      q->pipe.parse_cd = c->pipe.parse_cd; q->pipe.parse_wu = c->pipe.parse_wu; q->pipe.mf_ts_min = c->pipe.mf_ts_min; q->pipe.mf_ts_mul = c->pipe.mf_ts_mul; q->tile = c->tile; q->pipe.sa_exact = c->pipe.sa_exact;
+      q->pipe.parse_cd = c->pipe.parse_cd; q->tile = c->tile;
       c->peers.push_back(q);
    }
    return c->peers[k - 1];
 }
 
 static size_t multi_chunk_blocks(size_t nblocks, int ndev) {
-   static const int forced = getenv("ZULTRA_CUDA_CHUNK_BLOCKS") ? atoi(getenv("ZULTRA_CUDA_CHUNK_BLOCKS")) : 0;
-   if (forced > 0) return (size_t)forced;
    size_t g = nblocks / ((size_t)ndev * 4);
    return g < 1 ? 1 : (g > 8 ? 8 : g);
 }
@@ -385,7 +254,7 @@ static int run_multi(zultra_cuda_ctx_t *c, int ndev, const uint8_t *host_hist, i
       c->counters[3] += p.stat_redo; c->counters[7] += p.stat_tiles;
    }
    c->ms[6] = tot.lap(); c->ms[7] = t_prep + c->ms[6];
-   c->counters[4] = g_zb_launches - l0; c->counters[5] = 1; c->counters[6] = ndev;
+   c->counters[4] = g_zb_launches - l0; c->counters[6] = ndev;
    return 0;
 }
 
@@ -409,10 +278,6 @@ int zultra_cuda_compress_blocks(zultra_cuda_ctx_t *c, const unsigned char *hist,
       cudaSetDevice(c->device);
       { char msg[64]; snprintf(msg, sizeof msg, "compress_blocks: end, devices %d", nd); zb_trace(msg, c->ms); }
       return ctx_leave(c, rc);
-   }
-   {
-      const int nl = lanes_wanted(c, n, clamp_block(block));
-      if (nl > 1) return ctx_leave(c, run_lanes(c, nl, hist, hist_size, in, 0, n, clamp_block(block), finalize, in_bits, flags, checksum, out, 0, out_cap, out_bits));
    }
    ZbStreamIn s = {in, n, hist, (uint32_t)hist_size, finalize, in_bits, checksum ? *checksum : 0};
    ZbRunOpts o;
@@ -473,10 +338,6 @@ int zultra_cuda_compress_blocks_device(zultra_cuda_ctx_t *c, const void *dev_in,
    int rc = ctx_enter(c);
    if (rc) return rc;
    if (!dev_in || !dev_out || !out_bits) return ZULTRA_CUDA_ERR_ARG;
-   {
-      const int nl = lanes_wanted(c, n, clamp_block(block));
-      if (nl > 1) return ctx_leave(c, run_lanes(c, nl, 0, 0, 0, (const uint8_t *)dev_in, n, clamp_block(block), finalize, 0, flags, checksum, 0, (uint8_t *)dev_out, out_cap, out_bits));
-   }
    ZbStreamIn s = {0, n, 0, 0, finalize, 0, checksum ? *checksum : 0};
    ZbRunOpts o;
    o.dev_in = (const uint8_t *)dev_in; o.dev_out = (uint8_t *)dev_out; o.dev_out_cap = out_cap;
@@ -708,10 +569,9 @@ int zultra_cuda_window_sa_lcp(zultra_cuda_ctx_t *c, const unsigned char *win, in
    ZbStreamIn s = {win, (size_t)n, 0, 0, 1, 0, 0};
    ZbRunOpts o; ZbDump d; o.dump = &d; o.stop_after = 1;
    std::vector<ZbStreamRes> res;
-   const bool was_exact = c->pipe.sa_exact;
    c->pipe.sa_exact = true;                          /* the parity artefact is the exact suffix array */
    rc = run_one(c, s, 2097152u + 65536u, o, res);   /* one window: block size above any window */
-   c->pipe.sa_exact = was_exact;
+   c->pipe.sa_exact = false;
    if (rc == 0) memcpy(words, d.sa_lcp.data(), (size_t)n * 4);
    return ctx_leave(c, rc ? ZULTRA_CUDA_ERR_CUDA : 0);
 }

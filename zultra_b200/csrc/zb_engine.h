@@ -41,7 +41,6 @@ struct ZbRunOpts {
    ZbDump *dump = 0;
    int stop_after = 99;            /* 1 = SA, 2 = match (stage dumps) */
    float ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};   /* h2d, sa, match, greedy+split, parse, emit, d2h, total */
-   double t_abs[8] = {0, 0, 0, 0, 0, 0, 0, 0};   /* host clock (ms since an arbitrary origin) at the end of each stage: lane timelines */
 };
 
 /* main positions per match-finder tile: as large as shared memory allows (amortises the 32768 look-back entries every
@@ -154,24 +153,24 @@ static inline int zb_run_batch(ZbPipe &p, const ZbStreamIn *s, int ns, uint32_t 
       size_t at = 0;
       for (int i = 0; i < ns; i++) { zb_h2d(p.st, p.in.p + at, s[i].data - s[i].hist_len, s[i].hist_len + s[i].n); at += s[i].hist_len + s[i].n; }
    }
-   zb_sync(p.st); o.ms[0] = tm.lap(); o.t_abs[0] = zb_now_ms();
+   zb_sync(p.st); o.ms[0] = tm.lap();
    if (zb_failed()) return -3;      /* allocation or copy failed: nothing has been launched on missing buffers */
    p.stage_sa();
-   zb_sync(p.st); o.ms[1] = tm.lap(); o.t_abs[1] = zb_now_ms();
+   zb_sync(p.st); o.ms[1] = tm.lap();
    if (zb_failed()) return -3;
    if (o.stop_after >= 2) {
       p.stage_match(o.tile_main ? o.tile_main : zb_pick_tile(total_block));
-      zb_sync(p.st); o.ms[2] = tm.lap(); o.t_abs[2] = zb_now_ms();
+      zb_sync(p.st); o.ms[2] = tm.lap();
       if (zb_failed()) return -3;
    }
    if (o.stop_after >= 3) {
       p.stage_greedy();
       if (zb_failed()) return -3;
       p.stage_split();
-      zb_sync(p.st); o.ms[3] = tm.lap(); o.t_abs[3] = zb_now_ms();
+      zb_sync(p.st); o.ms[3] = tm.lap();
       if (zb_failed()) return -3;
       p.stage_parse();
-      zb_sync(p.st); o.ms[4] = tm.lap(); o.t_abs[4] = zb_now_ms();
+      zb_sync(p.st); o.ms[4] = tm.lap();
       if (zb_failed()) return -3;
       p.stage_emit_prepare();
       if (zb_failed()) return -3;
@@ -188,7 +187,7 @@ static inline int zb_run_batch(ZbPipe &p, const ZbStreamIn *s, int ns, uint32_t 
          o.phase_maps.assign((size_t)ns * 8, 0);
          p.phase_maps(so, o.phase_maps.data());
          memcpy(o.phase_bits, o.phase_maps.data(), sizeof(o.phase_bits));
-         zb_sync(p.st); o.ms[5] = tm.lap(); o.ms[7] = tot.lap(); o.t_abs[5] = zb_now_ms();
+         zb_sync(p.st); o.ms[5] = tm.lap(); o.ms[7] = tot.lap();
          return zb_failed() ? -3 : 0;
       }
       p.stage_emit_finish(so);
@@ -279,17 +278,6 @@ static inline int zb_finish_chunks(ZbPipe &p, const unsigned *in_bits, size_t *o
    zb_sync(p.st);
    if (zb_failed()) return -3;
    for (size_t i = 0; i < so.size(); i++) { out_off[i] = (size_t)p.h_sout[i].out_word_off * 4; bits[i] = p.h_sout[i].total_bits; }
-   return 0;
-}
-/* lane of a stream that shares one output buffer with the other lanes: abs_bits = absolute bit offset of the lane's first
-   bit in ext_words (zeroed by the caller); edge words are merged with atomicOr by the emitters */
-static inline int zb_finish_lane(ZbPipe &p, unsigned long long abs_bits, uint32_t *ext_words, unsigned long long *end_bits) {
-   std::vector<ZbStreamOut> so(1);
-   memset(&so[0], 0, sizeof(ZbStreamOut));
-   so[0].first_win = 0; so[0].nwin = (uint32_t)p.nwin; so[0].in_bits = abs_bits;
-   p.stage_emit_finish(so, ext_words);
-   zb_sync(p.st);
-   *end_bits = p.h_sout[0].total_bits;
    return 0;
 }
 #endif

@@ -93,12 +93,12 @@ ZB_HD void zb_tok_count(const uint8_t *T, uint32_t p, uint32_t len, uint32_t off
    else lc[T[p]] += sign;
 }
 
-/* Warm-up of a parse chunk whose candidates read at most `reach` positions past its end: the configured warm-up WU is the
+/* Warm-up of a parse chunk whose candidates read at most `reach` positions past its end: the full warm-up ZB_WU is the
    258-position horizon plus a settling margin; the same margin above `reach` (stage_parse, D2). */
-ZB_HD int zb_warmup_len(int WU, int reach) {
-   const int margin = WU > ZB_MAX_MATCH ? WU - ZB_MAX_MATCH : 0;
-   const int w = reach + margin;
-   return w < WU ? w : WU;
+static_assert(ZB_WU > ZB_MAX_MATCH, "the adaptive warm-up needs a settling margin above the 258-position horizon");
+ZB_HD int zb_warmup_len(int reach) {
+   const int w = reach + (ZB_WU - ZB_MAX_MATCH);
+   return w < ZB_WU ? w : ZB_WU;
 }
 
 template <class T> struct ZbBuf {
@@ -215,8 +215,7 @@ struct ZbPipe {
    int nsub = 0;
    /* stats */
    bool sa_exact = false;       /* run the suffix sort to the end (stage dumps); see stage_sa */
-   int parse_cd = 0, parse_wu = ZB_WU;   /* parse chunk (0 = by batch size, see stage_parse) / warm-up positions */
-   int mf_ts_min = ZB_TS_MIN, mf_ts_mul = ZB_TS_MUL;   /* rank walk -> text walk switch (zb_mf_scan) */
+   int parse_cd = 0;            /* parse chunk (0 = by batch size, see stage_parse) */
    int stat_sa_rounds = 0, stat_redo = 0, stat_ub = 0, stat_tiles = 0;
    double t_stage[8];
 
@@ -230,9 +229,7 @@ struct ZbPipe {
    void stage_parse();
    void stage_emit(const std::vector<ZbStreamOut> &streams) { stage_emit_prepare(); stage_emit_finish(streams); }
    void stage_emit_prepare();                                   /* path, token bits, sub-block sizes: independent of the bit phase */
-   /* stitch scan for the entering phase, then emission.  ext_words != 0: write into that zeroed word buffer, every stream's
-      in_bits being its ABSOLUTE bit offset there (lanes of one stream sharing one output, zb_capi.cu) */
-   void stage_emit_finish(const std::vector<ZbStreamOut> &streams, uint32_t *ext_words = 0);
+   void stage_emit_finish(const std::vector<ZbStreamOut> &streams);   /* stitch scan for the entering phase, then emission */
    void phase_maps(const std::vector<ZbStreamOut> &streams, unsigned long long *bits_out);   /* per stream: total bits for each entering phase 0..7 */
    std::vector<ZbStreamOut> plan;   /* streams of a prepared (phase 1) batch, for the emit call that follows */
    /* checksum partials of byte ranges of the device input: kind 1 = Adler-32, 2 = CRC-32 */
@@ -309,10 +306,6 @@ inline void ZbPipe::stage_sa() {
    if (zb_failed()) return;      /* fail fast: no launch ever sees a missing buffer (zb_run_batch reports the error) */
    int wb = 0; while ((1L << wb) < nwin) wb++;
    int nbytes = (64 - wb) / 8; if (nbytes > 7) nbytes = 7;
-   {  /* development knob: fewer key bytes = fewer radix passes over all suffixes, more suffixes left to the doubling rounds */
-      static const int nb_env = getenv("ZULTRA_CUDA_SA_NBYTES") ? atoi(getenv("ZULTRA_CUDA_SA_NBYTES")) : 0;
-      if (nb_env >= 3 && nb_env < nbytes) nbytes = nb_env;
-   }
    const uint8_t *T = in_ptr; const ZbWinDesc *wd = win.p; const uint32_t *wbs = wbase.p; const int nw = nwin;
    uint64_t *kA = keyA.p; uint32_t *vA = valA.p;
    zb_tag("sa_keys");
@@ -932,14 +925,12 @@ inline void ZbPipe::stage_match(uint32_t tile_main) {
 #endif
 #ifndef ZB_EMU
       if (g_zb_prof_on) { zb_tag("mf_scan"); zb_prof_begin(0, st); }
-      zb_mf_scan_k<<<cnt, ZB_MF_THREADS, smem, st>>>(td, first, unit_words.p, unit_cnt.p, ivb, qstride, stride, tq, mt, gl, go, wbs, tile_main, mf_ts_min, mf_ts_mul);
+      /* ZB_TS_MIN / ZB_TS_MUL go in as arguments: compiled in as constants the kernel ran 3 % slower on B200 */
+      zb_mf_scan_k<<<cnt, ZB_MF_THREADS, smem, st>>>(td, first, unit_words.p, unit_cnt.p, ivb, qstride, stride, tq, mt, gl, go, wbs, tile_main, ZB_TS_MIN, ZB_TS_MUL);
       if (g_zb_prof_on) zb_prof_end(st);
       if (g_zb_prof_on) { zb_tag("mf_text"); zb_prof_begin(0, st); }
-      {  /* a 16384-position tile has twice the queue and 49 KB of text (4 CTAs per SM): twice the warps per CTA keep the SM as full */
-         static const int mt_thr = getenv("ZULTRA_CUDA_MT_THREADS") ? atoi(getenv("ZULTRA_CUDA_MT_THREADS")) : 0;
-         const int thr = (mt_thr == 256 || mt_thr == 512) ? mt_thr : (tile_main > 8192 ? 512 : 256);
-         zb_mf_text_k<<<cnt, thr, smem_txt, st>>>(td, first, ivb, qstride, tq, mt, gl, go, wbs, wdp, Tp);
-      }
+      /* a 16384-position tile has twice the queue and 49 KB of text (4 CTAs per SM): twice the warps per CTA keep the SM as full */
+      zb_mf_text_k<<<cnt, tile_main > 8192 ? 512 : 256, smem_txt, st>>>(td, first, ivb, qstride, tq, mt, gl, go, wbs, wdp, Tp);
       if (g_zb_prof_on) zb_prof_end(st);
       zb_count_launch(2);
       ZB_CUDA_CHECK(cudaGetLastError());
@@ -1791,7 +1782,7 @@ __global__ void __launch_bounds__(256) zb_choice_k(long npch, const ZbSub *sb, c
  * u16 pairing) - short matches (< 40) only look 39 positions ahead - and every cost is also streamed to a global scratch row
  * ([step][thread], so a warp's store is one 64-byte line) from which the rare far reads of leave-alone matches (>= 40: one
  * cost, up to 258 ahead) and the two 259-entry signatures are taken.  A chunk starts from cost 0 and a step adds at most 15
- * bits, so with CD + WU <= 4368 steps the u16 costs never wrap and are compared as plain integers.
+ * bits, so with CD + ZB_WU <= 4368 steps the u16 costs never wrap and are compared as plain integers.
  * The candidate lengths of all short matches of a position share ONE prefix-minimum sweep: key = (cost[i + k] + lencost(k))
  * << 6 | 63 - k, one multiply-add and one minimum per length (the length cost and the tie-break come pre-combined out of a
  * per-sub-block table), the sweep pausing at every match's length to price that match.
@@ -1824,7 +1815,6 @@ __device__ __forceinline__ void zb_dp_signature(int16_t *__restrict__ dst, size_
 /* positions [lo, from) of one chunk, descending; t = step of position from - 1 on entry.  All per-step addresses are running
    pointers (the cost row advances by one row, the records / text / choices retreat by one element, the ring slot by one slot
    modulo 64): the loop is instruction bound, and 64-bit address arithmetic from the position index was a fifth of it. */
-template <int UNR>
 __device__ __forceinline__ void zb_dp_range(const uint8_t *__restrict__ T, const uint4 *__restrict__ cand, const ZbDpTab *__restrict__ tab, int lo, int from,
                                             uint32_t *__restrict__ choice, uint16_t *ring0, uint16_t *far0, int &t_io, uint32_t &cprev_io, const bool KEEP) {
    const int NT = ZB_DP_THREADS;
@@ -1869,7 +1859,7 @@ __device__ __forceinline__ void zb_dp_range(const uint8_t *__restrict__ T, const
                const int ml = (int)((e >> 5) & 63u);
                while (k <= ml) {
                   const int kstop = ml < kw - 1 ? ml : kw - 1;
-#pragma unroll UNR
+#pragma unroll 2
                   for (; k <= kstop; k++, pr -= NT) {
                      const uint32_t key = ((uint32_t)*pr << 6) + lenkey[k - ZB_MIN_MATCH];
                      curmin = key < curmin ? key : curmin;
@@ -1895,10 +1885,10 @@ __device__ __forceinline__ void zb_dp_range(const uint8_t *__restrict__ T, const
    t_io = t; cprev_io = cprev;
 }
 
-template <int UNR, int MINB>
-__global__ void __launch_bounds__(ZB_DP_THREADS, MINB) zb_parse_dp_k(const ZbSub *sb, const ZbSubTabs *tb, const uint32_t *dcs, long ndch, int pass, const ZbWinDesc *wd,
-                                                               const uint32_t *wbs, const uint8_t *T, const uint4 *cand, uint32_t *bm, int16_t *sgt, int16_t *sgw,
-                                                               size_t SS, uint16_t *far, int CD, int WU, int nslot, const int *reach) {
+/* unroll 2 of the sweep at 7 CTAs per SM (62 registers) measured fastest on B200 */
+__global__ void __launch_bounds__(ZB_DP_THREADS, 7) zb_parse_dp_k(const ZbSub *sb, const ZbSubTabs *tb, const uint32_t *dcs, long ndch, int pass, const ZbWinDesc *wd,
+                                                            const uint32_t *wbs, const uint8_t *T, const uint4 *cand, uint32_t *bm, int16_t *sgt, int16_t *sgw,
+                                                            size_t SS, uint16_t *far, int CD, int nslot, const int *reach) {
    extern __shared__ __align__(16) uint8_t zb_dp_sm[];
    uint16_t *ring_s = (uint16_t *)zb_dp_sm;                                   /* [ZB_NR][ZB_DP_THREADS] */
    ZbDpTab *tab_s = (ZbDpTab *)(zb_dp_sm + ZB_NR * ZB_DP_THREADS * 2);        /* [nslot] */
@@ -1925,18 +1915,18 @@ __global__ void __launch_bounds__(ZB_DP_THREADS, MINB) zb_parse_dp_k(const ZbSub
    const int lo = (int)(s.ps + k * CD);
    const int hi = (int)(lo + CD < (int)s.pe ? lo + CD : (int)s.pe);
    const int end = (int)s.pe;
-   /* adaptive warm-up (reach != 0): the chunk only reads costs up to `reach` positions past its end, so only those have to be
-      right, and the warm-up is the settling margin above THEM instead of above the full 258-position horizon */
-   const int rc = reach ? reach[c] : ZB_MAX_MATCH;
-   int from = hi + zb_warmup_len(WU, rc); if (from > end) from = end;
-   uint16_t *far0 = far + (size_t)blockIdx.x * (size_t)(CD + WU) * ZB_DP_THREADS + threadIdx.x;
+   /* adaptive warm-up: the chunk only reads costs up to `reach` positions past its end, so only those have to be right, and
+      the warm-up is the settling margin above THEM instead of above the full 258-position horizon */
+   const int rc = reach[c];
+   int from = hi + zb_warmup_len(rc); if (from > end) from = end;
+   uint16_t *far0 = far + (size_t)blockIdx.x * (size_t)(CD + ZB_WU) * ZB_DP_THREADS + threadIdx.x;
    int16_t *sw = sgw + (size_t)c, *sg = sgt + (size_t)c;
    int step = 0; uint32_t cprev = 0;
    /* warm-up [hi, from) then the chunk [lo, hi): ONE copy of the recurrence (the two phases as iterations of a loop that is
       not unrolled) - the kernel is instruction-issue bound and its code should stay inside the I-cache */
 #pragma unroll 1
    for (int phase = 0; phase < 2; phase++) {
-      zb_dp_range<UNR>(t, cand + gb, tab, phase ? lo : hi, phase ? hi : from, bm + gb, ring0, far0, step, cprev, phase != 0);
+      zb_dp_range(t, cand + gb, tab, phase ? lo : hi, phase ? hi : from, bm + gb, ring0, far0, step, cprev, phase != 0);
       zb_dp_signature(phase ? sg : sw, SS, far0, phase ? lo : hi, from, end, step, cprev, phase == 0, phase ? ZB_MAX_MATCH : rc);
    }
 }
@@ -1975,8 +1965,7 @@ struct ZbDwShared {            /* per warp */
    records stay the same.  The walker tracks the stretch of identical records it is in (whole blocks of 32), tests that
    periodicity once the stretch is 517 positions long, and from then on copies 32 choices per step instead of scanning them -
    a 64 KiB run of a mozilla-shaped input is one serial chain of 128 chunks, and this chain is what the repair's time is. */
-struct ZbDwUni { uint4 ra, rb; uint32_t rl, delta; int len, top; bool periodic; int aE; bool a_valid;      /* pch[j] = choice of position aE + 1 + j, while a_valid */
-                 int n_copy, n_scan, n_slow; /* positions done by each path (ZULTRA_CUDA_FIX_DEBUG) */ };
+struct ZbDwUni { uint4 ra, rb; uint32_t rl, delta; int len, top; bool periodic; int aE; bool a_valid; };   /* pch[j] = choice of position aE + 1 + j, while a_valid */
 
 __device__ __forceinline__ void zb_dw_run(const uint8_t *__restrict__ t, const zb_match_t *__restrict__ match, int lo, int from, int end,
                                           zb_match_t *__restrict__ best, ZbDwShared &sh, int &slot, ZbDwUni &U, const int lane,
@@ -2077,7 +2066,7 @@ __device__ __forceinline__ void zb_dw_run(const uint8_t *__restrict__ t, const z
                wide = true;
                i0 -= 128;
                s += 128; if (s >= ZB_DW_RING) s -= ZB_DW_RING;
-               U.len += 128; U.n_copy += 128;
+               U.len += 128;
                na = ya[0]; nb = yb[0]; nl = yl[0];
 #pragma unroll
                for (int k = 0; k < 3; k++) { ca[k] = ya[k + 1]; cb[k] = yb[k + 1]; cl[k] = yl[k + 1]; }
@@ -2103,7 +2092,7 @@ __device__ __forceinline__ void zb_dw_run(const uint8_t *__restrict__ t, const z
          s += nb_pos; if (s >= ZB_DW_RING) s -= ZB_DW_RING;
          __syncwarp();
          base = ring[s];
-         U.len += nb_pos; U.n_copy += nb_pos;
+         U.len += nb_pos;
          i0 -= 32;
          continue;
       }
@@ -2171,7 +2160,6 @@ __device__ __forceinline__ void zb_dw_run(const uint8_t *__restrict__ t, const z
          }
          base = (base + (uint32_t)__shfl_sync(0xffffffffu, r, nb_pos - 1)) & 0xffffu;
          s += nb_pos; if (s >= ZB_DW_RING) s -= ZB_DW_RING;
-         U.n_scan += nb_pos;
          ZB_DW_STRETCH();
          i0 -= 32;
          continue;
@@ -2247,7 +2235,6 @@ __device__ __forceinline__ void zb_dw_run(const uint8_t *__restrict__ t, const z
          __syncwarp();
       }
       if (lane < nb_pos) ((uint32_t *)best)[i0 - lane] = outw;
-      U.n_slow += nb_pos;
       ZB_DW_STRETCH();
       i0 -= 32;
    }
@@ -2261,7 +2248,7 @@ __device__ __forceinline__ void zb_dw_run(const uint8_t *__restrict__ t, const z
    verifies again afterwards, so a race with a neighbouring run costs a round, never correctness. */
 __global__ void __launch_bounds__(ZB_DW_THREADS) zb_parse_fix_k(const ZbSub *sb, const ZbSubTabs *tb, const uint32_t *dcs, const uint32_t *badlist, int nbad, const uint8_t *ok,
                                                                 const ZbWinDesc *wd, const uint32_t *wbs, const uint8_t *T, const zb_match_t *mt, zb_match_t *bm,
-                                                                int16_t *sgt, int16_t *sgw, size_t SS, int CD, long long *dbg, const int *reach) {
+                                                                int16_t *sgt, int16_t *sgw, size_t SS, int CD, const int *reach) {
    __shared__ ZbDwShared sh_all[ZB_DW_WARPS];
    const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
    const long g = (long)blockIdx.x * ZB_DW_WARPS + wi;
@@ -2278,8 +2265,7 @@ __global__ void __launch_bounds__(ZB_DW_THREADS) zb_parse_fix_k(const ZbSub *sb,
    zb_match_t *b0 = bm + gb;
    const int end = (int)s.pe;
    int slot = 0;
-   ZbDwUni U; U.ra = make_uint4(0u, 0u, 0u, 0u); U.rb = U.ra; U.rl = 0; U.delta = 0; U.len = 0; U.top = -1; U.periodic = false; U.aE = 0; U.a_valid = false; U.n_copy = U.n_scan = U.n_slow = 0;
-   const long long clk0 = clock64();
+   ZbDwUni U; U.ra = make_uint4(0u, 0u, 0u, 0u); U.rb = U.ra; U.rl = 0; U.delta = 0; U.len = 0; U.top = -1; U.periodic = false; U.aE = 0; U.a_valid = false;
    {
       const uint32_t *src = (const uint32_t *)&tb[x].cost; uint32_t *dstw = (uint32_t *)&sh.tab;
       for (int e = lane; e < (int)(sizeof(ZbCostTab) / 4); e += 32) dstw[e] = src[e];
@@ -2308,7 +2294,7 @@ __global__ void __launch_bounds__(ZB_DW_THREADS) zb_parse_fix_k(const ZbSub *sb,
       int16_t *sw = sgw + (size_t)nx;
       if (ok_nx) {      /* (inside a run of wrong chunks nx is redone whatever it had assumed: no reason to wait for its 259 loads) */
          bool same = true;
-         const int lim = reach ? reach[nx] : ZB_MAX_MATCH;      /* nx reads no cost further out (adaptive warm-up, stage_parse) */
+         const int lim = reach[nx];      /* nx reads no cost further out (adaptive warm-up, stage_parse) */
          int16_t got[(ZB_MAX_MATCH + 32) / 32];
 #pragma unroll
          for (int j = 0; j < (ZB_MAX_MATCH + 32) / 32; j++) { const int e = lane + 32 * j; got[j] = e <= lim ? sw[(size_t)e * SS] : (int16_t)0; }      /* all in flight together */
@@ -2330,7 +2316,6 @@ __global__ void __launch_bounds__(ZB_DW_THREADS) zb_parse_fix_k(const ZbSub *sb,
       c = nx;
       __syncwarp();
    }
-   if (dbg && lane == 0) { long long *d = dbg + 5 * g; d[0] = U.n_copy; d[1] = U.n_scan; d[2] = U.n_slow; d[3] = clock64() - clk0; d[4] = badlist[g]; }
 }
 #endif
 
@@ -2414,8 +2399,7 @@ inline void ZbPipe::stage_parse() {
    const uint32_t CPv = (uint32_t)cp;
    if (cd_auto < 128) cd_auto = 128;      /* small inputs (one 48 KB stream, a GPU's share of a strongly scaled 51 MB): short chunks = short serial chains, the warm-up then dominates a chunk */
    if (cd_auto > ZB_CD) cd_auto = ZB_CD;
-   int WU = parse_wu; if (WU > 2048) WU = 2048;
-   int CD = parse_cd ? parse_cd : cd_auto; if (CD > 2048) CD = 2048;      /* CD + WU <= 4368: u16 costs cannot wrap (zb_parse_dp_k) */
+   int CD = parse_cd ? parse_cd : cd_auto; if (CD > 2048) CD = 2048;      /* CD + ZB_WU <= 4368: u16 costs cannot wrap (zb_parse_dp_k) */
    const int ns = nsub;
    ZbSub *sb = sub.p; ZbSubTabs *tb = tabs.p; uint32_t *cn = counters.p;
    ZbGreedyView gv = {ph.p, wintbase.p, wtokbase.p, tokpos.p, wbase.p, glen.p, goff.p, in_ptr, win.p};
@@ -2488,7 +2472,7 @@ inline void ZbPipe::stage_parse() {
    pentry.need(npch + 1); pbits.need(npch + 1);
 #ifndef ZB_EMU
    exitc.need((size_t)(npch + 1) * ZB_EXROW);
-   dpfar.need((size_t)((ndch + ZB_DP_THREADS - 1) / ZB_DP_THREADS) * (size_t)(CD + WU + 8) * ZB_DP_THREADS + 64);   
+   dpfar.need((size_t)((ndch + ZB_DP_THREADS - 1) / ZB_DP_THREADS) * (size_t)(CD + ZB_WU + 8) * ZB_DP_THREADS + 64);
 #endif
    if (zb_failed()) return;
    uint32_t *dcs = dchunk_sub.p, *pcs = pchunk_sub.p;
@@ -2507,10 +2491,8 @@ inline void ZbPipe::stage_parse() {
       need(c) = max(reach(c), need(c - 1) - CD) - then every entry any comparison or repair start ever uses is either inside a
       verified chunk or inside the verified part of a warm-up zone (induction from the exact last chunk of the sub-block).
       The lists do not change over the passes: once per batch, 8 tasks of 33 positions per chunk. */
-   const int awu_env = getenv("ZULTRA_CUDA_PARSE_AWU") ? atoi(getenv("ZULTRA_CUDA_PARSE_AWU")) : 1;      /* read per call: the tests flip it */
-   const bool awu = awu_env && WU > ZB_MAX_MATCH;
    int *rch = 0;
-   if (awu && ndch > 0) {
+   if (ndch > 0) {
       dreach.need(2 * (size_t)ndch + 2);
       if (zb_failed()) return;
       int *need = dreach.p;
@@ -2557,16 +2539,7 @@ inline void ZbPipe::stage_parse() {
    const size_t dp_smem = (size_t)ZB_NR * ZB_DP_THREADS * 2 + (size_t)dp_nslot * sizeof(ZbDpTab);
    {  /* the limit is a per-function global: always the largest configuration, so concurrent host threads cannot undercut each other */
       const size_t smax = (size_t)ZB_NR * ZB_DP_THREADS * 2 + (size_t)ZB_DP_THREADS * sizeof(ZbDpTab);
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<4, 9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<1, 9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<2, 9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<4, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<2, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<1, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<2, 12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<2, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<4, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
-      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k<2, 7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
+      ZB_CUDA_CHECK(cudaFuncSetAttribute(zb_parse_dp_k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smax));
    }
    if (npch > 0) {
       if (g_zb_prof_on) { zb_tag("parse_cand"); zb_prof_begin(0, st); }
@@ -2582,21 +2555,13 @@ inline void ZbPipe::stage_parse() {
 
    for (int pass = 0; pass < 4; pass++) {
       /* D2: chunked backward recurrence.  Chunk k of a sub-block covers [ps + k*CD, ..).  Every chunk but the last
-         starts WU positions past its end from an all-zero cost guess; the relative costs it sees at its own end
+         starts up to ZB_WU positions past its end from an all-zero cost guess; the relative costs it sees at its own end
          (sig_warm) are later compared with what the next chunk really computed there (sig_true). */
 #ifndef ZB_EMU
       if (ndch > 0) {
          if (g_zb_prof_on) { zb_tag("parse_dp"); zb_prof_begin(0, st); }
-         {
-            const unsigned grid = (unsigned)((ndch + ZB_DP_THREADS - 1) / ZB_DP_THREADS);
-            /* development variants (ZULTRA_CUDA_DP_VAR): k-loop unroll factor x CTAs per SM asked of the compiler */
-            static const int var = getenv("ZULTRA_CUDA_DP_VAR") ? atoi(getenv("ZULTRA_CUDA_DP_VAR")) : 0;
-#define ZB_DP_LAUNCH(U_, B_) zb_parse_dp_k<U_, B_><<<grid, ZB_DP_THREADS, dp_smem, st>>>(sb, tb, dcs, ndch, pass, wd, wbs, T, (const uint4 *)cand.p, (uint32_t *)bm, sgt, sgw, SS, dpfar.p, CD, WU, dp_nslot, rch)
-            if (var == 1) ZB_DP_LAUNCH(1, 9); else if (var == 2) ZB_DP_LAUNCH(2, 9); else if (var == 3) ZB_DP_LAUNCH(4, 10); else if (var == 4) ZB_DP_LAUNCH(2, 10); else if (var == 5) ZB_DP_LAUNCH(1, 10);
-            else if (var == 6) ZB_DP_LAUNCH(2, 12); else if (var == 7) ZB_DP_LAUNCH(4, 9); else if (var == 8) ZB_DP_LAUNCH(2, 6); else if (var == 9) ZB_DP_LAUNCH(4, 6);
-            else if (var == 10) ZB_DP_LAUNCH(2, 9); else ZB_DP_LAUNCH(2, 7);      /* measured on B200: unroll 2 at 62 registers (8 CTAs per SM) */
-#undef ZB_DP_LAUNCH
-         }
+         zb_parse_dp_k<<<(unsigned)((ndch + ZB_DP_THREADS - 1) / ZB_DP_THREADS), ZB_DP_THREADS, dp_smem, st>>>(sb, tb, dcs, ndch, pass, wd, wbs, T, (const uint4 *)cand.p, (uint32_t *)bm,
+                                                                                                       sgt, sgw, SS, dpfar.p, CD, dp_nslot, rch);
          if (g_zb_prof_on) zb_prof_end(st);
          zb_count_launch(1);
          ZB_CUDA_CHECK(cudaGetLastError());
@@ -2608,7 +2573,6 @@ inline void ZbPipe::stage_parse() {
          const ZbSub s = sb[dcs[c]];
          if (pass > 0 && !s.is_dyn) return;
          if (emu_lean) {
-            if (c == 0 && pass == 0 && getenv("ZB_EMU_DP_LEAN")[0] == '2') fprintf(stderr, "parse: compact candidate record path\n");
             const uint32_t kc = (uint32_t)c - s.dchunk_base;
             const uint32_t gb = wbs[s.win];
             const uint8_t *t = T + wd[s.win].in_off;
@@ -2616,7 +2580,7 @@ inline void ZbPipe::stage_parse() {
             const int lo = (int)(s.ps + kc * CD);
             const int hi = (int)(lo + CD < (int)s.pe ? lo + CD : (int)s.pe);
             const int end = (int)s.pe;
-            int from = hi + zb_warmup_len(WU, rch ? rch[c] : ZB_MAX_MATCH); if (from > end) from = end;
+            int from = hi + zb_warmup_len(rch[c]); if (from > end) from = end;
             const ZbCostTab &ct = tb[dcs[c]].cost;
             std::vector<uint32_t> v((size_t)(from - lo) + 1, 0u);      /* cost of step tt (position from - 1 - tt) */
             uint32_t cprev = 0;
@@ -2651,7 +2615,7 @@ inline void ZbPipe::stage_parse() {
          const int lo = (int)(s.ps + k * CD);
          const int hi = (int)(lo + CD < (int)s.pe ? lo + CD : (int)s.pe);
          const int end = (int)s.pe;
-         int from = hi + zb_warmup_len(WU, rch ? rch[c] : ZB_MAX_MATCH); if (from > end) from = end;
+         int from = hi + zb_warmup_len(rch[c]); if (from > end) from = end;
          ZbRingLocal ring;
          for (int i = 0; i < ZB_RING; i++) ring.v[i] = 0;
          int slot = 0;
@@ -2683,7 +2647,7 @@ inline void ZbPipe::stage_parse() {
          neighbour's costs; repeat until nothing disagrees.  By induction from the (exact) last chunk of each sub-block the
          fixed point is the sequential result; the number of rounds is the longest run of consecutive wrong chunks
          (non-resynchronising data such as long byte runs), independent chains repair concurrently. */
-      for (int round = 0;; round++) {
+      for (;;) {
          zb_memset(st, cn + 7, 0, 4);
          zb_tag("parse_verify");
          zb_launch(st, ndch, ZB_LAMBDA(long c) {
@@ -2692,7 +2656,7 @@ inline void ZbPipe::stage_parse() {
             const uint32_t k = (uint32_t)c - s.dchunk_base;
             if (!(pass > 0 && !s.is_dyn) && k + 1 < s.ndchunk) {
                const int16_t *a = sgw + (size_t)c, *b = sgt + (size_t)(c + 1);
-               const int lim = rch ? rch[c] : ZB_MAX_MATCH;      /* the chunk reads no cost further out */
+               const int lim = rch[c];      /* the chunk reads no cost further out */
                for (int q = 0; q <= lim && good; q++) if (a[(size_t)q * SS] != b[(size_t)q * SS]) good = 0;
             }
             ok[c] = good;
@@ -2702,30 +2666,9 @@ inline void ZbPipe::stage_parse() {
          zb_d2h(st, &nbad, cn + 7, 4); zb_sync(st);
          if (!nbad) break;
          stat_redo += (int)nbad;
-#ifdef ZB_EMU
-         if (getenv("ZB_DUMP_BAD") && round == 0) {   /* analysis aid of the host build: which chunks failed to re-synchronise */
-            for (uint32_t e = 0; e < nbad; e++) {
-               const ZbSub &s = sb[dcs[bad[e]]];
-               fprintf(stderr, "BAD pass %d win %u pos %u sub [%u,%u)\n", pass, s.win, s.ps + (bad[e] - s.dchunk_base) * CD, s.ps, s.pe);
-            }
-         }
-#endif
 #ifndef ZB_EMU
          if (g_zb_prof_on) { zb_tag("parse_repair"); zb_prof_begin(0, st); }
-         static const int fix_dbg = getenv("ZULTRA_CUDA_FIX_DEBUG") ? atoi(getenv("ZULTRA_CUDA_FIX_DEBUG")) : 0;
-         long long *dbgp = 0;
-         if (fix_dbg) { scratch.need((size_t)nbad * 10 + 64); dbgp = (long long *)scratch.p; zb_memset(st, dbgp, 0, (size_t)nbad * 40); }
-         zb_parse_fix_k<<<(unsigned)((nbad + ZB_DW_WARPS - 1) / ZB_DW_WARPS), ZB_DW_THREADS, 0, st>>>(sb, tb, dcs, bad, (int)nbad, ok, wd, wbs, T, mt, bm, sgt, sgw, SS, CD, dbgp, rch);
-         if (fix_dbg) {
-            std::vector<long long> hd((size_t)nbad * 5);
-            zb_d2h(st, hd.data(), dbgp, hd.size() * 8); zb_sync(st);
-            std::vector<int> idx; for (int e = 0; e < (int)nbad; e++) if (hd[5 * (size_t)e + 3]) idx.push_back(e);
-            std::sort(idx.begin(), idx.end(), [&](int a, int b) { return hd[5 * (size_t)a + 3] > hd[5 * (size_t)b + 3]; });
-            long long tc = 0, tn = 0, ts = 0; for (int e : idx) { tc += hd[5 * (size_t)e]; tn += hd[5 * (size_t)e + 1]; ts += hd[5 * (size_t)e + 2]; }
-            fprintf(stderr, "fix pass %d round %d: %u bad chunks, %zu chains; positions copy %lld scan %lld slow %lld\n", pass, round, nbad, idx.size(), tc, tn, ts);
-            for (size_t q = 0; q < idx.size() && q < 6; q++) { const long long *d = &hd[5 * (size_t)idx[q]]; const ZbSub *unused = 0; (void)unused;
-               fprintf(stderr, "   chain at chunk %lld: copy %lld scan %lld slow %lld cycles %lld\n", d[4], d[0], d[1], d[2], d[3]); }
-         }
+         zb_parse_fix_k<<<(unsigned)((nbad + ZB_DW_WARPS - 1) / ZB_DW_WARPS), ZB_DW_THREADS, 0, st>>>(sb, tb, dcs, bad, (int)nbad, ok, wd, wbs, T, mt, bm, sgt, sgw, SS, CD, rch);
          if (g_zb_prof_on) zb_prof_end(st);
          zb_count_launch(1);
          ZB_CUDA_CHECK(cudaGetLastError());
@@ -3099,7 +3042,7 @@ inline void ZbPipe::phase_maps(const std::vector<ZbStreamOut> &streams, unsigned
    }
 }
 
-inline void ZbPipe::stage_emit_finish(const std::vector<ZbStreamOut> &streams, uint32_t *ext_words) {
+inline void ZbPipe::stage_emit_finish(const std::vector<ZbStreamOut> &streams) {
    const uint32_t CPv = (uint32_t)cp;
    const int ns = nsub;
    ZbSub *sb = sub.p; ZbSubTabs *tb = tabs.p; uint32_t *cn = counters.p;
@@ -3152,18 +3095,13 @@ inline void ZbPipe::stage_emit_finish(const std::vector<ZbStreamOut> &streams, u
    });
    zb_d2h(st, h_sout.data(), so, sizeof(ZbStreamOut) * nstr); zb_sync(st);
    /* output area: every stream gets a zeroed, word-aligned span */
-   if (ext_words) {
-      for (int q = 0; q < nstr; q++) h_sout[q].out_word_off = 0;
-      zb_h2d(st, so, h_sout.data(), sizeof(ZbStreamOut) * nstr);
-   } else {
-      uint64_t w = 0;
-      for (int q = 0; q < nstr; q++) { h_sout[q].out_word_off = w; w += (h_sout[q].total_bits + 31) / 32 + 2; }
-      out.need(w + 4);
-      if (zb_failed()) return;
-      zb_memset(st, out.p, 0, (w + 4) * 4);
-      zb_h2d(st, so, h_sout.data(), sizeof(ZbStreamOut) * nstr);
-   }
-   uint32_t *ow = ext_words ? ext_words : out.p;
+   uint64_t w = 0;
+   for (int q = 0; q < nstr; q++) { h_sout[q].out_word_off = w; w += (h_sout[q].total_bits + 31) / 32 + 2; }
+   out.need(w + 4);
+   if (zb_failed()) return;
+   zb_memset(st, out.p, 0, (w + 4) * 4);
+   zb_h2d(st, so, h_sout.data(), sizeof(ZbStreamOut) * nstr);
+   uint32_t *ow = out.p;
    /* E4: tokens */
    zb_tag("emit_tokens");
    zb_launch(st, npch, ZB_LAMBDA(long c) {

@@ -62,8 +62,7 @@ template <class F> static inline void zb_launch_(int line, zb_stream_t st, long 
    if (n <= 0) { zb_tag(0); return; }
    /* few tasks are the serial per-sub-block / per-node ones (Huffman builds, splitter scans): give each its own warp, so that
       32 unrelated control flows do not serialise inside one, and its own SM share instead of crowding two SMs */
-   static const long heavy_max = getenv("ZULTRA_CUDA_HEAVY_SINGLE_MAX") ? atol(getenv("ZULTRA_CUDA_HEAVY_SINGLE_MAX")) : 4096;
-   if (n <= (blk == 64 ? heavy_max : 4096)) blk = 1;   /* blk == 64 marks the heavy serial tasks at their call sites */
+   if (n <= 4096) blk = 1;
    if (g_zb_prof_on) zb_prof_begin(line, st);
    zb_task_kernel<<<(unsigned)((n + blk - 1) / blk), blk, 0, st>>>(n, f);
    if (g_zb_prof_on) zb_prof_end(st);
