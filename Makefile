@@ -9,7 +9,7 @@ B = build
 
 all: zultra_b200/libzultra_b200.so zultra_b200/zultra
 
-$(B)/%.o: $(CS)/%.cu $(CS)/zb_core.h $(CS)/zb_rt.h $(CS)/zb_pipeline.h $(CS)/zb_engine.h include/zultra_cuda.h
+$(B)/%.o: $(CS)/%.cu $(CS)/zb_core.h $(CS)/zb_rt.h $(CS)/zb_pipeline.h $(CS)/zb_engine.h include/zultra_cuda.h include/libzultra.h
 	@mkdir -p $(B)
 	$(NVCC) $(NVFLAGS) -c $< -o $@
 
@@ -24,7 +24,7 @@ zultra_b200/zultra: $(B)/zultra_cli.o zultra_b200/libzultra_b200.so
 	$(CC) -o $@ $(B)/zultra_cli.o -Lzultra_b200 -lzultra_b200 -lz -Wl,-rpath,'$$ORIGIN'
 
 emu:
-	g++ -O2 -g -DZB_EMU -std=c++17 -fPIC -shared -I$(CS) -o tests/emu/libzb_emu.so tests/emu/zb_emu.cpp tests/emu/zb_prims_emu.cpp
+	g++ -O2 -g -DZB_EMU -std=c++17 -fPIC -shared -I$(CS) -o tests/emu/libzb_emu.so tests/emu/zb_emu.cpp tests/emu/zb_batch_dict_emu.cpp tests/emu/zb_prims_emu.cpp
 
 oracle:
 	$(MAKE) -C oracle all

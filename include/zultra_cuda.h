@@ -99,6 +99,15 @@ int zultra_cuda_stitch_device(zultra_cuda_ctx_t *pCtx, void *pDevDst, int nParts
 int zultra_cuda_memory_compress_batch(zultra_cuda_ctx_t *pCtx, const unsigned char *const *ppInData, const size_t *pnInSizes,
                                       unsigned char *const *ppOutData, const size_t *pnMaxOutSizes, size_t *pnOutSizes, size_t nStreams,
                                       unsigned int nFlags, unsigned int nMaxBlockSize);
+/* Same, every stream compressed against one preset dictionary: stream i equals zultra_stream_init(nFlags, nMaxBlockSize),
+   zultra_stream_set_dictionary(pDictionaryData, nDictionaryDataSize), then payload i with ZULTRA_FINALIZE.  The dictionary's
+   last min(size, 32768) bytes are the history of each payload's first max-block; zlib framing writes the FDICT header with
+   the DICTID (Adler-32 of the whole dictionary), 4 bytes more than zultra_memory_bound allows for; the trailer checksum covers
+   the payload only.  The dictionary crosses the bus once per call, the payloads packed.  NULL / 0 = no dictionary (the
+   output of zultra_cuda_memory_compress_batch); a negative size, or NULL with a size above 0, is ZULTRA_CUDA_ERR_ARG. */
+int zultra_cuda_memory_compress_batch_dict(zultra_cuda_ctx_t *pCtx, const unsigned char *const *ppInData, const size_t *pnInSizes,
+                                           unsigned char *const *ppOutData, const size_t *pnMaxOutSizes, size_t *pnOutSizes, size_t nStreams,
+                                           unsigned int nFlags, unsigned int nMaxBlockSize, const void *pDictionaryData, int nDictionaryDataSize);
 
 /* Checksums on the device for device-resident input (frame.c:74 Adler-32, frame.c:324 CRC-32). */
 int zultra_cuda_checksum_device(zultra_cuda_ctx_t *pCtx, const void *pDevData, size_t nSize, unsigned int nFlags, unsigned int *pnChecksum);

@@ -61,6 +61,8 @@ def load():
         L.zultra_cuda_checksum_combine.restype = C.c_uint
         L.zultra_cuda_checksum_combine.argtypes = [C.c_uint, C.c_uint, C.c_uint, C.c_ulonglong]
         L.zultra_cuda_memory_compress_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint, C.c_uint]
+        L.zultra_cuda_memory_compress_batch_dict.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint, C.c_uint,
+                                                             C.c_void_p, C.c_int]
         L.zultra_cuda_window_sa_lcp.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.zultra_cuda_window_matches.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_uint]
         L.zultra_cuda_block_stages.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -255,23 +257,31 @@ class CudaCtx:
         self.L.zultra_cuda_last_counters(self.p, v)
         return dict(zip(["windows", "sub_blocks", "sa_rounds", "parse_redo", "launches", "r5", "devices", "r7"], [int(x) for x in v]))
 
-    def memory_compress_batch(self, payloads, flags=ZULTRA_FLAG_ZLIB_FRAMING, block=0):
+    def memory_compress_batch(self, payloads, flags=ZULTRA_FLAG_ZLIB_FRAMING, block=0, dictionary=None):
+        """One stream per payload; None where the C call reports (size_t)-1.  With `dictionary`, every payload is compressed
+        against that preset dictionary (zultra_cuda_memory_compress_batch_dict), as a Stream with set_dictionary would."""
         n = len(payloads)
         arrs = [_u8(p) for p in payloads]
-        caps = [memory_bound(len(a), flags, block) for a in arrs]
+        d = _u8(dictionary) if dictionary is not None else None
+        # zlib framing with a dictionary: the 4-byte DICTID, which zultra_memory_bound does not count (neither does the reference's)
+        dictid = 4 if d is not None and len(d) and (flags & 3) == ZULTRA_FLAG_ZLIB_FRAMING else 0
+        caps = [memory_bound(len(a), flags, block) + dictid for a in arrs]
         outs = [np.empty(c, dtype=np.uint8) for c in caps]
         inp = (C.c_void_p * n)(*[a.ctypes.data for a in arrs]); ins = (C.c_size_t * n)(*[len(a) for a in arrs])
         outp = (C.c_void_p * n)(*[o.ctypes.data for o in outs]); oc = (C.c_size_t * n)(*caps); osz = (C.c_size_t * n)()
-        rc = self.L.zultra_cuda_memory_compress_batch(self.p, inp, ins, outp, oc, osz, n, flags, block)
+        if d is None:
+            rc = self.L.zultra_cuda_memory_compress_batch(self.p, inp, ins, outp, oc, osz, n, flags, block)
+        else:
+            rc = self.L.zultra_cuda_memory_compress_batch_dict(self.p, inp, ins, outp, oc, osz, n, flags, block, d.ctypes.data if len(d) else None, len(d))
         if rc != 0:
-            raise RuntimeError("zultra_cuda_memory_compress_batch failed: %d" % rc)
+            raise RuntimeError("zultra_cuda_memory_compress_batch%s failed: %d" % ("" if d is None else "_dict", rc))
         bad = C.c_size_t(-1).value
         return [None if osz[i] == bad else outs[i][: osz[i]].tobytes() for i in range(n)]
 
 
-def memory_compress_batch(payloads, flags=ZULTRA_FLAG_ZLIB_FRAMING, block=0, device=-1):
+def memory_compress_batch(payloads, flags=ZULTRA_FLAG_ZLIB_FRAMING, block=0, device=-1, dictionary=None):
     ctx = CudaCtx(device)
     try:
-        return ctx.memory_compress_batch(payloads, flags, block)
+        return ctx.memory_compress_batch(payloads, flags, block, dictionary=dictionary)
     finally:
         ctx.close()

@@ -3,6 +3,7 @@
  */
 #include "zb_engine.h"
 #include "../../include/zultra_cuda.h"
+#include "../../include/libzultra.h"
 #include <new>
 #include <mutex>
 #include <thread>
@@ -476,36 +477,38 @@ void zultra_cuda_release_cached(void) {
    g_pool.clear();
 }
 
-/* frame bytes written on the host side of the batch call (frame.c:387-452, :509-547) */
-static size_t put_header(unsigned char *o, unsigned flags) {
-   if (flags & 2) { const unsigned char h[10] = {0x1f, 0x8b, 8, 0, 0, 0, 0, 0, 2, 255}; memcpy(o, h, 10); return 10; }
-   if (flags & 1) { o[0] = 0x78; o[1] = 0xda; return 2; }
-   return 0;
-}
-static size_t put_footer(unsigned char *o, unsigned flags, unsigned ck, unsigned long long n) {
-   if (flags & 2) { for (int i = 0; i < 4; i++) { o[i] = (unsigned char)(ck >> (8 * i)); o[4 + i] = (unsigned char)(n >> (8 * i)); } return 8; }
-   if (flags & 1) { for (int i = 0; i < 4; i++) o[i] = (unsigned char)(ck >> (8 * (3 - i))); return 4; }
-   return 0;
-}
-
 int zultra_cuda_memory_compress_batch(zultra_cuda_ctx_t *c, const unsigned char *const *in, const size_t *in_sizes, unsigned char *const *outp,
                                       const size_t *out_caps, size_t *out_sizes, size_t nstreams, unsigned int flags, unsigned int block) {
+   return zultra_cuda_memory_compress_batch_dict(c, in, in_sizes, outp, out_caps, out_sizes, nstreams, flags, block, 0, 0);
+}
+
+int zultra_cuda_memory_compress_batch_dict(zultra_cuda_ctx_t *c, const unsigned char *const *in, const size_t *in_sizes, unsigned char *const *outp,
+                                           const size_t *out_caps, size_t *out_sizes, size_t nstreams, unsigned int flags, unsigned int block,
+                                           const void *dict, int dict_size) {
+   if (!c || dict_size < 0 || (!dict && dict_size > 0)) return ZULTRA_CUDA_ERR_ARG;
    int rc = ctx_enter(c);
    if (rc) return rc;
    block = clamp_block(block);
    long long l0 = g_zb_launches;
-   const unsigned hdr = (flags & 2) ? 10 : ((flags & 1) ? 2 : 0), ftr = (flags & 2) ? 8 : ((flags & 1) ? 4 : 0);
+   /* the dictionary's last 32 KiB are the first window's history of every stream (libzultra.c:250-253); the frame header, with
+      the DICTID of the whole dictionary under zlib framing, is the same for every stream and built once (frame.c) */
+   const uint32_t dk = dict_size > 0 ? (uint32_t)std::min(dict_size, ZB_HISTORY) : 0u;
+   const uint8_t *dtail = dk ? (const uint8_t *)dict + (dict_size - (int)dk) : 0;
+   unsigned char hdr_bytes[16];
+   const int hn = zultra_frame_encode_header(hdr_bytes, (int)sizeof(hdr_bytes), flags, dk ? dict : 0, dk ? dict_size : 0);
+   if (hn < 0) return ctx_leave(c, ZULTRA_CUDA_ERR_ARG);
+   const size_t hdr = (size_t)hn, ftr = (size_t)zultra_frame_get_footer_size(flags);
    float ms[8] = {0};
    size_t i0 = 0;
    while (i0 < nstreams) {
-      /* sub-batch: bounded positions */
+      /* sub-batch: bounded window bytes (every stream's dictionary history counts) */
       size_t i1 = i0, bytes = 0;
       std::vector<ZbStreamIn> s;
-      while (i1 < nstreams && (i1 == i0 || bytes + in_sizes[i1] + ((in_sizes[i1] / block) * ZB_HISTORY) < ((size_t)768 << 20))) {
+      while (i1 < nstreams && (i1 == i0 || bytes + dk + in_sizes[i1] + ((in_sizes[i1] / block) * ZB_HISTORY) < ((size_t)768 << 20))) {
          if (in_sizes[i1] > 0) {   /* empty input yields (size_t)-1 like the reference (libzultra.c:275,617) */
-            ZbStreamIn t = {in[i1], in_sizes[i1], 0, 0, 1, 0, (flags & 2) ? 0u : 1u};
+            ZbStreamIn t = {in[i1], in_sizes[i1], dtail, dk, 1, 0, (flags & 2) ? 0u : 1u};
             s.push_back(t);
-            bytes += in_sizes[i1] + (in_sizes[i1] / block) * ZB_HISTORY;
+            bytes += dk + in_sizes[i1] + (in_sizes[i1] / block) * ZB_HISTORY;
          }
          i1++;
       }
@@ -513,6 +516,7 @@ int zultra_cuda_memory_compress_batch(zultra_cuda_ctx_t *c, const unsigned char 
       ZbRunOpts o;
       o.checksum_kind = (flags & 2) ? 2 : ((flags & 1) ? 1 : 0);
       o.want_out_ptr = 1;
+      o.shared_hist = dk ? 1 : 0;
       c->pipe.counters.need(64);
       zb_memset(c->pipe.st, c->pipe.counters.p, 0, 64 * 4);
       if (!s.empty() && zb_run_batch(c->pipe, s.data(), (int)s.size(), block, c->out, res, o)) return ctx_leave(c, ZULTRA_CUDA_ERR_CUDA);
@@ -528,9 +532,10 @@ int zultra_cuda_memory_compress_batch(zultra_cuda_ctx_t *c, const unsigned char 
                const size_t nb = (size_t)((res[k].total_bits + 7) / 8);
                if (hdr + nb + ftr > out_caps[i]) out_sizes[i] = (size_t)-1;
                else {
-                  size_t w = put_header(outp[i], flags);
-                  memcpy(outp[i] + w, obase + res[k].out_off, nb); w += nb;
-                  w += put_footer(outp[i] + w, flags, res[k].checksum, in_sizes[i]);
+                  memcpy(outp[i], hdr_bytes, hdr);
+                  memcpy(outp[i] + hdr, obase + res[k].out_off, nb);
+                  size_t w = hdr + nb;
+                  w += (size_t)zultra_frame_encode_footer(outp[i] + w, (int)ftr, res[k].checksum, (long long)in_sizes[i], flags);
                   out_sizes[i] = w;
                }
             }

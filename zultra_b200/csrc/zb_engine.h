@@ -31,6 +31,9 @@ struct ZbRunOpts {
    int dev_offsets = 0;            /* dev_in holds several streams (chunks of one resident buffer): ZbStreamIn::dev_off locates each */
    int direct_h2d = 0;             /* several streams from host memory, each [history | data] contiguous there: one DMA per stream straight from the
                                       caller's buffer instead of gathering them into page-locked staging first */
+   int shared_hist = 0;            /* several streams from host memory with the SAME history (s[i].hist and hist_len equal: a preset
+                                      dictionary): gather and send the history once and the payloads packed, then build every
+                                      stream's [history | data] on the device (stage_assemble) */
    int phase = 3;                  /* 1 = stop after the phase-independent part (shards), 2 = only finish, 3 = both */
    unsigned long long phase_bits[8] = {0, 0, 0, 0, 0, 0, 0, 0};
    std::vector<unsigned long long> phase_maps;   /* phase 1: 8 entries per stream (phase_bits = those of stream 0) */
@@ -68,37 +71,46 @@ static inline int zb_run_batch(ZbPipe &p, const ZbStreamIn *s, int ns, uint32_t 
    size_t in_bytes = 0;
    for (int i = 0; i < ns; i++) in_bytes += s[i].hist_len + s[i].n;
    if (in_bytes >= ((size_t)1 << 31)) return -1;
+   /* shared history: the staged input is [history | payload 0 | payload 1 | ...] (stage_assemble expands it on the device) */
+   const bool shared = o.shared_hist && !o.dev_in && ns > 0;
+   const uint32_t sh_len = shared ? s[0].hist_len : 0;
+   for (int i = 0; i < ns && shared; i++) if (s[i].hist_len != sh_len || s[i].hist != s[0].hist) return -1;
+   size_t stage_bytes = shared ? sh_len : in_bytes;
+   for (int i = 0; i < ns && shared; i++) stage_bytes += s[i].n;
    ZbTimer tm, tot;
    /* copy straight from the caller's buffer when [history | data] is contiguous there; otherwise gather the streams into
       page-locked memory (several host threads: a single memcpy stream does not keep up with the DMA that follows) */
-   const bool single_direct = (ns == 1 && !o.dev_in && (s[0].hist_len == 0 || s[0].hist + s[0].hist_len == s[0].data));
-   bool multi_direct = ns > 1 && !o.dev_in && o.direct_h2d;
+   const bool single_direct = (ns == 1 && !o.dev_in && !shared && (s[0].hist_len == 0 || s[0].hist + s[0].hist_len == s[0].data));
+   bool multi_direct = ns > 1 && !o.dev_in && !shared && o.direct_h2d;
    for (int i = 0; i < ns && multi_direct; i++) if (s[i].hist_len && s[i].hist + s[i].hist_len != s[i].data) multi_direct = false;
    uint8_t *stage = 0;
-   bool staged_to_device = false, pipe_fail = false;      /* the gather threads already sent the staged input to p.in */
+   bool staged_to_device = false, pipe_fail = false;      /* the gather threads already sent the staged input to the device */
    if (!o.dev_in && !single_direct && !multi_direct) {
-      p.hin.need(in_bytes + 16);
+      p.hin.need(stage_bytes + 16);
       stage = p.hin.p;
       if (!stage || zb_failed()) return -3;
-      std::vector<size_t> offs(ns + 1, 0);
-      for (int i = 0; i < ns; i++) offs[i + 1] = offs[i] + s[i].hist_len + s[i].n;
-      const int nth = in_bytes > ((size_t)8 << 20) ? 4 : 1;
+      std::vector<size_t> offs(ns + 1, sh_len);      /* where stream i's staged bytes start */
+      for (int i = 0; i < ns; i++) offs[i + 1] = offs[i] + (shared ? 0 : s[i].hist_len) + s[i].n;
+      const int nth = stage_bytes > ((size_t)8 << 20) ? 4 : 1;
 #ifndef ZB_EMU
       /* large batches: every gathering thread sends what it has gathered to the device in 4 MiB pieces on its own stream, so the
          DMA runs under the remaining memcpys instead of after them (347 MB of small streams: 25 ms of gather + DMA -> the longer of the two) */
       const bool piped = nth > 1 && p.stager.init();
-      if (piped) { p.in.need(in_bytes + 16); if (zb_failed()) return -3; staged_to_device = true; }
+      ZbBuf<uint8_t> &dev_stage = shared ? p.pk : p.in;
+      if (piped) { dev_stage.need(stage_bytes + 16); if (zb_failed()) return -3; staged_to_device = true; }
 #else
       const bool piped = false;
 #endif
       auto gather = [&](int a, int b, int lane) {
-         size_t sent = a < ns ? offs[a] : in_bytes;
+         size_t sent = a == 0 ? 0 : (a < ns ? offs[a] : stage_bytes);
+         if (shared && a == 0 && b > 0) memcpy(stage, s[0].hist, sh_len);      /* the history once, ahead of the first payload */
          for (int i = a; i < b; i++) {
-            if (s[i].hist_len) memcpy(stage + offs[i], s[i].hist, s[i].hist_len);
-            memcpy(stage + offs[i] + s[i].hist_len, s[i].data, s[i].n);
+            const size_t h = shared ? 0 : s[i].hist_len;
+            if (h) memcpy(stage + offs[i], s[i].hist, h);
+            memcpy(stage + offs[i] + h, s[i].data, s[i].n);
 #ifndef ZB_EMU
             if (piped && (offs[i + 1] - sent >= ((size_t)4 << 20) || i + 1 == b)) {
-               cudaMemcpyAsync(p.in.p + sent, stage + sent, offs[i + 1] - sent, cudaMemcpyHostToDevice, p.stager.st[lane]);
+               cudaMemcpyAsync(dev_stage.p + sent, stage + sent, offs[i + 1] - sent, cudaMemcpyHostToDevice, p.stager.st[lane]);
                sent = offs[i + 1];
             }
 #endif
@@ -114,7 +126,7 @@ static inline int zb_run_batch(ZbPipe &p, const ZbStreamIn *s, int ns, uint32_t 
          int a = 0;
          for (int k = 0; k < nth; k++) {   /* equal byte shares */
             int b = a;
-            while (b < ns && (k == nth - 1 || offs[b] < in_bytes / nth * (k + 1))) b++;
+            while (b < ns && (k == nth - 1 || offs[b] < stage_bytes / nth * (k + 1))) b++;
             th.emplace_back(gather, a, b, k);
             a = b;
          }
@@ -148,10 +160,18 @@ static inline int zb_run_batch(ZbPipe &p, const ZbStreamIn *s, int ns, uint32_t 
    for (int i = 0; i < ns; i++) res[i].checksum = s[i].checksum;
    if (wins.empty()) { out.clear(); return 0; }
    if (pipe_fail) return -3;
-   p.setup(wins, o.dev_in ? o.dev_in : (single_direct ? s[0].data - s[0].hist_len : (staged_to_device ? (const uint8_t *)0 : stage)), in_bytes, o.dev_in != 0);
+   p.setup(wins, o.dev_in ? o.dev_in : (single_direct ? s[0].data - s[0].hist_len : ((staged_to_device || shared) ? (const uint8_t *)0 : stage)), in_bytes, o.dev_in != 0);
    if (multi_direct && !zb_failed()) {      /* setup allocated the device input (no source given): one DMA per stream */
       size_t at = 0;
       for (int i = 0; i < ns; i++) { zb_h2d(p.st, p.in.p + at, s[i].data - s[i].hist_len, s[i].hist_len + s[i].n); at += s[i].hist_len + s[i].n; }
+   }
+   if (shared && !zb_failed()) {      /* the packed input (already on the device when the gather sent it) -> [history | data] per stream */
+      if (!staged_to_device) { p.pk.need(stage_bytes + 16); if (zb_failed()) return -3; zb_h2d(p.st, p.pk.p, stage, stage_bytes); }
+      std::vector<uint32_t> tab(2 * (size_t)ns + 2);
+      size_t a = 0, q = sh_len;
+      for (int i = 0; i < ns; i++) { tab[2 * i] = (uint32_t)a; tab[2 * i + 1] = (uint32_t)q; a += sh_len + s[i].n; q += s[i].n; }
+      tab[2 * (size_t)ns] = (uint32_t)a; tab[2 * (size_t)ns + 1] = (uint32_t)q;
+      p.stage_assemble(tab, sh_len, in_bytes);
    }
    zb_sync(p.st); o.ms[0] = tm.lap();
    if (zb_failed()) return -3;      /* allocation or copy failed: nothing has been launched on missing buffers */

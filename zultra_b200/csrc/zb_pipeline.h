@@ -189,6 +189,7 @@ struct ZbPipe {
    ZbBuf<ZbWinDesc> win; ZbBuf<uint32_t> wbase;
    ZbBuf<uint8_t> in;           /* device input (owned copy) */
    const uint8_t *in_ptr = 0;   /* input actually used by the stages (in.p or a caller's device buffer) */
+   ZbBuf<uint8_t> pk; ZbBuf<uint32_t> asm_tab;   /* shared-history batches: packed input and its stream table (stage_assemble) */
    /* suffix array stage */
    ZbBuf<uint64_t> keyA, keyB; ZbBuf<uint32_t> valA, valB, rank, sa, actA, actB, tmpA, tmpB, scratch;
    ZbBuf<uint32_t> sa_lcp;      /* packed SA|LCP words, rank order, per window at wbase[w] */
@@ -222,6 +223,7 @@ struct ZbPipe {
    void release_all();
    /* stages */
    void setup(const std::vector<ZbWinDesc> &wins, const uint8_t *h_in, size_t in_bytes, bool in_is_device);
+   void stage_assemble(const std::vector<uint32_t> &tab, uint32_t hist_len, size_t in_bytes);
    void stage_sa();
    void stage_match(uint32_t tile_main);
    void stage_greedy();
@@ -265,6 +267,55 @@ inline void ZbPipe::setup(const std::vector<ZbWinDesc> &wins, const uint8_t *h_i
       }
       in_ptr = in.p;
    }
+}
+
+/* ============================================================ shared-history input assembly ============================================================
+ * A batch whose streams all start from the same history (a preset dictionary, zultra_cuda_memory_compress_batch_dict) crosses
+ * the bus packed: pk = [history (hl bytes) | payload 0 | payload 1 | ...], the history once.  This pass writes the layout the
+ * stages read, [history | payload i] for every stream back to back in `in`, so the history is copied on the device and not on
+ * the host or the bus.  tab: {start in `in`, start of the payload in pk} per stream, then {total bytes, packed bytes}.
+ * One task per aligned 16 bytes of `in`: a task whose 16 bytes come from one run of pk (all but about two per stream) reads
+ * five aligned words, funnel-shifts them and stores one vector; a task across the history/payload seam or a stream end goes
+ * byte by byte.  Bytes past the total are written as zero (the buffer has 16 bytes of slack).
+ */
+inline void ZbPipe::stage_assemble(const std::vector<uint32_t> &h_tab, uint32_t hl, size_t in_bytes) {
+   const int ns = (int)h_tab.size() / 2 - 1;
+   asm_tab.need(h_tab.size());
+   if (zb_failed()) return;
+   zb_h2d(st, asm_tab.p, h_tab.data(), h_tab.size() * 4);
+   const uint32_t *tab = asm_tab.p; const uint8_t *src = pk.p; uint8_t *dst = in.p; const uint32_t total = (uint32_t)in_bytes;
+   zb_tag("batch_assemble");
+   zb_launch(st, (long)((in_bytes + 15) / 16), ZB_LAMBDA(long x) {
+      const uint32_t b0 = (uint32_t)x * 16u;
+      int lo = 0, hi = ns - 1;      /* the stream holding byte b0 */
+      while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (tab[2 * mid] <= b0) lo = mid; else hi = mid - 1; }
+      const uint32_t r = b0 - tab[2 * lo];
+      const uint32_t s0 = r < hl ? r : tab[2 * lo + 1] + (r - hl);
+      const uint32_t run = r < hl ? hl - r : tab[2 * lo + 2] - b0;      /* bytes from s0 on that are contiguous in pk */
+      uint32_t w[4];
+      if (run >= 16) {
+         const uint32_t *q = (const uint32_t *)(src + (s0 & ~3u)), sh = (s0 & 3u) * 8u;
+         uint32_t v[5];
+#pragma unroll
+         for (int k = 0; k < 5; k++) v[k] = q[k];
+#pragma unroll
+         for (int k = 0; k < 4; k++) w[k] = (uint32_t)((((uint64_t)v[k + 1] << 32) | v[k]) >> sh);
+      } else {
+         w[0] = w[1] = w[2] = w[3] = 0;
+         for (uint32_t j = 0, i = (uint32_t)lo; j < 16; j++) {
+            const uint32_t b = b0 + j;
+            if (b >= total) break;
+            while (b >= tab[2 * i + 2]) i++;
+            const uint32_t q = b - tab[2 * i];
+            w[j >> 2] |= (uint32_t)src[q < hl ? q : tab[2 * i + 1] + (q - hl)] << (8 * (j & 3));
+         }
+      }
+#ifdef __CUDA_ARCH__
+      *(uint4 *)(dst + b0) = make_uint4(w[0], w[1], w[2], w[3]);
+#else
+      memcpy(dst + b0, w, 16);
+#endif
+   }, 256);
 }
 
 /* ============================================================ suffix array + LCP ============================================================
@@ -3192,7 +3243,7 @@ inline void ZbPipe::release_all() {
 #ifndef ZB_EMU
    stager.release();
 #endif
-   win.release(); wbase.release(); in.release(); keyA.release(); keyB.release(); valA.release(); valB.release(); rank.release(); sa.release();
+   win.release(); wbase.release(); in.release(); pk.release(); asm_tab.release(); keyA.release(); keyB.release(); valA.release(); valB.release(); rank.release(); sa.release();
    actA.release(); actB.release(); tmpA.release(); tmpB.release(); scratch.release(); sa_lcp.release(); counters.release(); tiles.release();
    tile_iv.release(); tile_pd.release(); tile_cnt.release(); tile_q.release(); groups.release(); group_words.release(); group_cnt.release(); filt_seg.release(); units.release(); unit_words.release(); unit_cnt.release(); match.release(); glen.release(); goff.release(); exitoff.release(); exitc.release(); gentry.release();
    gtokcnt.release(); gtokbase.release(); tokpos.release(); wtok.release(); wtokbase.release(); wintbase.release(); ph.release();

@@ -244,6 +244,13 @@ def batch(count, seed=SEED_BATCH, lo=4096, hi=65536):
     return payloads
 
 
+def batch_dictionary(n, seed=SEED_BATCH):
+    """A preset dictionary for batch(count, seed): n bytes at a seeded offset of the text pool its text payloads are cut from."""
+    text_pool = enwik(4 << 20, seed=seed + 99)
+    o = int(np.random.default_rng(seed + 7).integers(0, len(text_pool) - n + 1))
+    return text_pool[o:o + n].copy()
+
+
 def lz_selftest(n, seed, alphabet, match_prob):
     """Data of the reference's self-test shape (tool/zultra.c:425-463): random literals over `alphabet` symbols mixed
     with copies of earlier data."""
